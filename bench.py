@@ -68,6 +68,8 @@ def parse_args():
     ap.add_argument("--two-pass", action="store_true", help="c5-slab: statistics pass + compress pass (two reads of the input) instead of the single-read path")
     ap.add_argument("--no-outlier-leg", action="store_true", help="skip the extra (reported, not headline) measurement with ~5%% outliers")
     ap.add_argument("--watchdog", type=int, default=1500, help="seconds after which a stuck run dumps every thread's Python stack to stderr and exits 3 (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step handed back (bin indices, DC, outliers and their "
+                                                          "count, [qtable,] scaling factor, reconstruction) as DIR/<name>.npy, rank 0 only")
     return ap.parse_args()
 
 
@@ -195,7 +197,31 @@ def make_sample(workload, n):
     return np.ascontiguousarray(x[:n]), qt
 
 
+DUMP_SAMPLE = 1 << 20  # elements kept of a longer output: at most 8 MiB an array, 20 MiB for the four long ones
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: name -> 1-D device tensor.  An array longer than DUMP_SAMPLE is cut to a seeded sample of its
+    positions, the same for every array of that length, so that the dumps of two builds compare element for element.
+    Floating-point arrays keep their type; the bin indices (uint8) are stored as float32.  An empty array is not written:
+    the outliers of a field that has none are absent, and n_outliers.npy holds their count."""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        if t.numel() == 0:
+            continue
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(SEED).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(path, f"{name}.npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float32))
+
+
 def main_reference(args):
+    if args.dump_outputs:
+        raise SystemExit("bench.py: --dump-outputs applies to the GPU arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
@@ -621,6 +647,13 @@ def main_ours(args):
     t_rt, t_c, t_d, t_k2, t_k1 = [float(v) for v in times.cpu()]
     a_last, c_last = pieces[-1]
     max_err = float((out[:c_last] - x[a_last:a_last + c_last]).abs().max().item())
+    if args.dump_outputs and rank == 0:
+        # with several sub-slabs per rank the outlier and output buffers hold the last sub-slab's
+        dumped = dict(bin_index=bins, dc=dc, ac=ac[:n_outs[-1]], n_outliers=torch.tensor([float(n_outs[-1])], dtype=torch.float64),
+                      sf=torch.tensor([sf], dtype=torch.float64), recon=out[:c_last])
+        if qt:
+            dumped["qtable"] = qtab
+        dump_outputs(args.dump_outputs, dumped)
     n_all = n_total if (strong and args.workload == "c5-slab") else n * world  # replicas / weak slabs: every rank's own elements
     gb_all = n_all * es * args.steps / 1e9
 

@@ -14,7 +14,7 @@ def test_two_ranks_over_nccl_from_c():
     import torch
 
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     exe = os.path.join(ROOT, "dctz_b200", "bin", "slab-comm-test")
     assert os.path.exists(exe), "run __graft_entry__.build()"
     p = subprocess.run([exe], capture_output=True, text=True, timeout=600)
