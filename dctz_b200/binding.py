@@ -24,6 +24,7 @@ EXPORTS = [
     "dctz_gpu_sf_from_max", "dctz_gpu_selftest_division", "dctz_gpu_launch_count", "dctz_gpu_compress_core_cb",
     "dctz_gpu_set_timing", "dctz_gpu_last_call_stats", "dctz_gpu_fused_phase_times", "dctz_gpu_compress_slab_comm",
     "dctz_gpu_sample_dev", "dctz_gpu_compress_spec_dev", "dctz_gpu_compress_spec_finish_dev",
+    "dctz_gpu_outlier_index_bytes", "dctz_gpu_outlier_index_dev", "dctz_gpu_decompress_ranges_dev",
 ]
 
 
@@ -78,6 +79,9 @@ def load_library():
         "dctz_gpu_compress_spec_finish_dev": (i32, [vp, vp, sz, sz, i32, dbl, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp]),
         "dctz_gpu_compress_field_dev": (i32, [vp, vp, sz, i32, dbl, i32, vp, vp, vp, vp, vp, vp, vp]),
         "dctz_gpu_decompress_dev": (i32, [vp, vp, vp, vp, u64, vp, sz, i32, dbl, dbl, i32, vp, vp, vp]),
+        "dctz_gpu_outlier_index_bytes": (sz, [sz]),
+        "dctz_gpu_outlier_index_dev": (i32, [vp, vp, sz, vp, vp, vp]),
+        "dctz_gpu_decompress_ranges_dev": (i32, [vp, vp, vp, vp, u64, vp, sz, i32, dbl, dbl, i32, vp, vp, sz, vp, vp, vp]),
         "dctz_gpu_scale_dev": (i32, [vp, vp, sz, i32, dbl, i32, vp]),
         "dctz_gpu_dct_blocks": (i32, [vp, vp, vp, sz, i32, i32, i32]),
         "dctz_gpu_dct64_dev": (i32, [vp, vp, vp, sz, i32, i32, i32, vp]),
@@ -332,6 +336,23 @@ class Context:
         mark more outliers than that"""
         self._check(self._lib.dctz_gpu_decompress_dev(self._h, d_bins, d_dc, d_ac or None, int(n_outliers), d_qtable or None, n, code,
                                                       float(eb), float(sf), int(bool(qt)), d_out, d_corrupt or None, stream or None))
+
+    def outlier_index_bytes(self, n):
+        """bytes of the outlier index of an n-element slab"""
+        return int(self._lib.dctz_gpu_outlier_index_bytes(int(n)))
+
+    def outlier_index_dev(self, d_bins, n, d_index, d_n_outliers=0, stream=0):
+        """build the outlier index of a slab's bin ids into d_index (outlier_index_bytes(n) bytes, 16-byte aligned);
+        d_n_outliers = optional device uint64 that receives the number of outliers the bin ids mark"""
+        self._check(self._lib.dctz_gpu_outlier_index_dev(self._h, d_bins, int(n), d_index, d_n_outliers or None, stream or None))
+
+    def decompress_ranges_dev(self, d_bins, d_dc, d_ac, n_outliers, d_qtable, n, code, eb, sf, qt, d_index, d_ranges, nranges, d_out,
+                              stream=0, d_corrupt=0):
+        """decode nranges {first, count} element ranges (uint64 pairs at d_ranges) into d_out, concatenated in range order;
+        d_corrupt = optional device uint32: bit 0 as in decompress_dev, bit 1 = a range outside [0, n) or of count 0"""
+        self._check(self._lib.dctz_gpu_decompress_ranges_dev(self._h, d_bins, d_dc, d_ac or None, int(n_outliers), d_qtable or None, int(n), code,
+                                                             float(eb), float(sf), int(bool(qt)), d_index, d_ranges, int(nranges), d_out,
+                                                             d_corrupt or None, stream or None))
 
     def scale_dev(self, d_x, n, code, sf, multiply, stream=0):
         self._check(self._lib.dctz_gpu_scale_dev(self._h, d_x, n, code, float(sf), int(bool(multiply)), stream or None))

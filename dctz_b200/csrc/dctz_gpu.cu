@@ -28,6 +28,7 @@
 
 #include "../../include/dctz_gpu.h"
 #include "fused.cuh"
+#include "ranges.cuh"
 
 using namespace dctz;
 
@@ -223,6 +224,9 @@ struct dctz_gpu_ctx {
   unsigned long long *d_dbg = nullptr;         // phase timestamps of the last single-launch kernels: [2][sm_count * 4][8]
   int dbg_grid[2] = {0, 0};
   int fused_stamps = 0;                        // DCTZ_FUSED_STAMPS=1: the single-launch kernels record their phase boundaries (dctz_gpu_fused_phase_times)
+  // region decompression (ranges.cuh)
+  int occ_ranges[2][2] = {};  // resident CTAs/SM of k_decompress_ranges [datatype][qt]
+  DevBuf region;              // [RangeCtl][piece_at, out_at: u64 per range][chunk_piece, chunk_out: u64 per 1024 ranges]
 };
 
 // ------------------------------------------------------------------------------------------
@@ -344,7 +348,7 @@ extern "C" void dctz_gpu_destroy(dctz_gpu_ctx *ctx) {
                    (void *)ctx->tb.thr_f, (void *)ctx->tb.sf_f};
   for (void *p : small) if (p) cudaFree(p);
   DevBuf *bufs[] = {&ctx->status, &ctx->slots, &ctx->qt_raw, &ctx->qt_j, &ctx->in, &ctx->bins, &ctx->dc, &ctx->ac,
-                    &ctx->qt, &ctx->qtraw, &ctx->out};
+                    &ctx->qt, &ctx->qtraw, &ctx->out, &ctx->region};
   for (DevBuf *b : bufs) if (b->p) cudaFree(b->p);
   for (double *p : ctx->d_dfrag) if (p) cudaFree(p);
   for (double *p : ctx->d_dfrag2) if (p) cudaFree(p);
@@ -461,6 +465,13 @@ static int ctx_init(dctz_gpu_ctx *ctx, int device) {
   ctx->occ_fused[1][1][1] = kernel_occupancy(k_decompress_fused<double, true>, DecompressCfg<double, true>::THREADS, DecompressCfg<double, true>::SMEM);
   ctx->occ_fused[1][0][0] = kernel_occupancy(k_decompress_fused<float, false>, DecompressCfg<float, false>::THREADS, DecompressCfg<float, false>::SMEM);
   ctx->occ_fused[1][0][1] = kernel_occupancy(k_decompress_fused<float, true>, DecompressCfg<float, true>::THREADS, DecompressCfg<float, true>::SMEM);
+  ctx->occ_ranges[1][0] = kernel_occupancy(k_decompress_ranges<double, false>, RangeCfg<double>::THREADS, RangeCfg<double>::SMEM);
+  ctx->occ_ranges[1][1] = kernel_occupancy(k_decompress_ranges<double, true>, RangeCfg<double>::THREADS, RangeCfg<double>::SMEM);
+  ctx->occ_ranges[0][0] = kernel_occupancy(k_decompress_ranges<float, false>, RangeCfg<float>::THREADS, RangeCfg<float>::SMEM);
+  ctx->occ_ranges[0][1] = kernel_occupancy(k_decompress_ranges<float, true>, RangeCfg<float>::THREADS, RangeCfg<float>::SMEM);
+  for (int b = 0; b < 2; b++)
+    for (int c = 0; c < 2; c++)
+      if (ctx->occ_ranges[b][c] < 1) return fail(ctx, DCTZ_GPU_ECUDA, "k_decompress_ranges [%d][%d] cannot be made resident", b, c);
   CU(cudaDeviceGetAttribute(&ctx->coop, cudaDevAttrCooperativeLaunch, device));
   CU(cudaMalloc(&ctx->d_barrier, 2 * sizeof(unsigned long long)));
   CU(cudaMemset(ctx->d_barrier, 0, 2 * sizeof(unsigned long long)));
@@ -1167,6 +1178,132 @@ extern "C" int dctz_gpu_decompress_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bins,
   }
   if (mode_qt) return launch_decompress<float, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, (float *)d_out, flag, st);
   return launch_decompress<float, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, (float *)d_out, flag, st);
+}
+
+// ------------------------------------------------------------------------------------------
+// region decompression (ranges.cuh, DESIGN.md §4.4)
+// ------------------------------------------------------------------------------------------
+// Outlier index of an N-element slab: [RegionIndexHdr (128 B)][group_prefix][chunk_prefix][counts], the arrays laid out as
+// scan_bufs lays them out in the context's scratch.
+struct RegionLayout { size_t ntiles, nchunks, off_gp, off_cp, off_counts, bytes; };
+static RegionLayout region_layout(size_t N) {
+  RegionLayout L;
+  L.ntiles = (N / BLK + WTILE - 1) / WTILE;
+  const size_t ngroups = (L.ntiles + 31) / 32;
+  L.nchunks = (ngroups + 1023) / 1024;
+  L.off_gp = 128;
+  L.off_cp = L.off_gp + up128(ngroups * 8);
+  L.off_counts = L.off_cp + up128(L.nchunks * 8);
+  L.bytes = L.off_counts + up128(L.ntiles * 4);
+  return L;
+}
+static_assert(sizeof(RegionIndexHdr) <= 128, "index header");
+
+extern "C" size_t dctz_gpu_outlier_index_bytes(size_t N) { return region_layout(N).bytes; }
+
+static RegionIndex region_view(const void *d_index, size_t N) {
+  const RegionLayout L = region_layout(N);
+  const char *p = (const char *)d_index;
+  RegionIndex v;
+  v.hdr = (const RegionIndexHdr *)p;
+  v.group_prefix = (const unsigned long long *)(p + L.off_gp);
+  v.chunk_prefix = (const unsigned long long *)(p + L.off_cp);
+  v.counts = (const unsigned *)(p + L.off_counts);
+  return v;
+}
+
+extern "C" int dctz_gpu_outlier_index_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bins, size_t N, void *d_index, uint64_t *d_n_outliers, void *stream) {
+  if (!ctx) return fail(nullptr, DCTZ_GPU_EINVAL, "ctx is NULL");
+  if (!d_bins || !d_index || N == 0) return fail(ctx, DCTZ_GPU_EINVAL, "outlier_index: NULL pointer or N == 0");
+  if (!aligned16(d_bins) || !aligned16(d_index)) return fail(ctx, DCTZ_GPU_EINVAL, "outlier_index: bin_index and the index must be 16-byte aligned");
+  if ((uintptr_t)d_n_outliers & 7u) return fail(ctx, DCTZ_GPU_EINVAL, "outlier_index: n_outliers must be 8-byte aligned");
+  const RegionLayout L = region_layout(N);
+  if (L.ntiles > 0xFFFFF000ull) return fail(ctx, DCTZ_GPU_EINVAL, "outlier_index: slab too large: %zu tiles", L.ntiles);
+  CU(cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  char *p = (char *)d_index;
+  RegionIndexHdr *hdr = (RegionIndexHdr *)p;
+  if (L.ntiles) {  // the decompress pre-pass, into the caller's buffer
+    unsigned *counts = (unsigned *)(p + L.off_counts);
+    FusedScan fused;
+    fused.out.group_prefix = (unsigned long long *)(p + L.off_gp);
+    fused.out.chunk_prefix = (unsigned long long *)(p + L.off_cp);
+    fused.out.done = ctx->d_done + 1;
+    fused.total = &hdr->n_full_outliers;
+    fused.n_entries = ((L.ntiles + 31) / 32 <= 1024) ? (unsigned)L.ntiles : 0u;  // small slab: the last CTA scans
+    const size_t want = (L.ntiles + 7) / 8;
+    const int grid = (int)(want < (size_t)ctx->sm_count * 16 ? want : (size_t)ctx->sm_count * 16);
+    k_count_bins<<<grid, 256, 0, st>>>(d_bins, N / BLK, counts, ctx->d_done + 3, fused);
+    ctx->launches++;
+    if (!fused.n_entries) {
+      k_scan_groups<<<(unsigned)L.nchunks, 1024, 0, st>>>(counts, (unsigned)L.ntiles, fused.out, fused.total);
+      ctx->launches++;
+    }
+  }
+  k_index_finish<<<1, 32, 0, st>>>(d_bins, N, (unsigned)L.ntiles, hdr, (unsigned long long *)d_n_outliers);
+  ctx->launches++;
+  CU(cudaGetLastError());
+  return DCTZ_GPU_OK;
+}
+
+template <typename T, bool QT>
+static int launch_ranges(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const float *d_dc, const float *d_ac, unsigned long long n_outliers, const T *d_qtable,
+                         size_t N, double eb, double sf, const void *d_index, const unsigned long long *d_ranges, size_t nranges, T *d_out,
+                         unsigned *flag, cudaStream_t st) {
+  typedef RangeCfg<T> Cfg;
+  const size_t nchunks = (nranges + 1023) / 1024;
+  const size_t off_ranges = 128, off_chunks = off_ranges + up128(nranges * 16);
+  TRY(grow(ctx, ctx->region, off_chunks + up128(nchunks * 16), true));  // (a new allocation starts zeroed: RangeCtl::done)
+  char *p = (char *)ctx->region.p;
+  RangePlan plan;
+  plan.ctl = (RangeCtl *)p;
+  plan.piece_at = (unsigned long long *)(p + off_ranges);
+  plan.out_at = plan.piece_at + nranges;
+  plan.chunk_piece = (unsigned long long *)(p + off_chunks);
+  plan.chunk_out = plan.chunk_piece + nchunks;
+  const RegionIndex idx = region_view(d_index, N);
+  k_range_plan<<<(unsigned)nchunks, 1024, 0, st>>>(d_ranges, nranges, N, idx.hdr, plan, flag);
+  ctx->launches++;
+  // the grid: every resident CTA, or fewer when the ranges cannot have that many pieces
+  const size_t ntiles = region_layout(N).ntiles;
+  const size_t max_pieces = nranges > PIECE_LIMIT / (ntiles + 1) ? (size_t)PIECE_LIMIT : nranges * (ntiles + 1);
+  const size_t resident = (size_t)ctx->sm_count * ctx->occ_ranges[sizeof(T) == 8][QT];
+  const size_t ctas = (max_pieces + Cfg::WARPS - 1) / Cfg::WARPS;
+  const int grid = (int)(ctas < resident ? ctas : resident);
+  const QtConsts<T> qk = make_qt<T>(eb);
+  const T bw = (sizeof(T) == 8) ? (T)(eb * 2 * 1.0) : (T)(float)((float)eb * 2 * 1.0);  // as launch_decompress
+  k_decompress_ranges<T, QT><<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(d_bins, d_dc, d_ac, d_qtable, N, bw, (T)sf, qk, idx, n_outliers, d_ranges, nranges,
+                                                                    plan, d_out, flag);
+  ctx->launches++;
+  CU(cudaGetLastError());
+  return DCTZ_GPU_OK;
+}
+
+extern "C" int dctz_gpu_decompress_ranges_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const float *d_dc, const float *d_ac, uint64_t n_outliers,
+                                              const void *d_qtable, size_t N, int datatype, double eb, double sf, int mode_qt, const void *d_index,
+                                              const uint64_t *d_ranges, size_t nranges, void *d_out, uint32_t *d_corrupt, void *stream) {
+  TRY(check_common(ctx, datatype, eb));
+  if (!d_bins || !d_dc || !d_index || !d_ranges || !d_out || N == 0 || nranges == 0 || (n_outliers && !d_ac))
+    return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: NULL pointer, N == 0 or no ranges");
+  if (mode_qt && !d_qtable) return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: QT mode needs the qtable");
+  const size_t es = datatype == DCTZ_GPU_DOUBLE ? 8 : 4;
+  if (!aligned16(d_bins) || !aligned16(d_index) || ((uintptr_t)d_ranges & 7u) || ((uintptr_t)d_out & (es - 1)))
+    return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: bin_index and the index must be 16-byte aligned, the ranges 8-byte, the output element-aligned");
+  if (((uintptr_t)d_dc & 3u) || ((uintptr_t)d_ac & 3u) || ((uintptr_t)d_qtable & (es - 1)))
+    return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: DC / AC_exact must be float-aligned, the qtable element-aligned");
+  if (!(sf > 0.0) || isinf(sf)) return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: scaling factor %g is not a positive finite number", sf);
+  if (nranges > ((size_t)1 << 40)) return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: %zu ranges", nranges);
+  if (region_layout(N).ntiles > 0xFFFFF000ull) return fail(ctx, DCTZ_GPU_EINVAL, "decompress_ranges: slab too large");
+  CU(cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  unsigned *flag = d_corrupt ? (unsigned *)d_corrupt : &ctx->d_ctl[1].corrupt;  // the caller's flag, else a scratch word nobody reads
+  const unsigned long long *rg = (const unsigned long long *)d_ranges;
+  if (datatype == DCTZ_GPU_DOUBLE) {
+    if (mode_qt) return launch_ranges<double, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sf, d_index, rg, nranges, (double *)d_out, flag, st);
+    return launch_ranges<double, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sf, d_index, rg, nranges, (double *)d_out, flag, st);
+  }
+  if (mode_qt) return launch_ranges<float, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, d_index, rg, nranges, (float *)d_out, flag, st);
+  return launch_ranges<float, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, d_index, rg, nranges, (float *)d_out, flag, st);
 }
 
 extern "C" int dctz_gpu_scale_dev(dctz_gpu_ctx *ctx, void *d_x, size_t N, int datatype, double sf, int multiply, void *stream) {

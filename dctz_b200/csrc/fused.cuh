@@ -427,7 +427,7 @@ k_decompress_fused(const uint8_t *__restrict__ bins, const float *__restrict__ d
   unsigned t0, t1;
   cta_tile_range(ntiles, &t0, &t1);
   const unsigned nt = t1 - t0;
-  for (int i = threadIdx.x; i < 256; i += Cfg::THREADS) center[i] = mul_rn<T>(mul_rn<T>((T)center_multiple((unsigned)i), bin_width), sf);
+  for (int i = threadIdx.x; i < 256; i += Cfg::THREADS) center[i] = center_coefficient<T>((unsigned)i, bin_width, sf);
   if (QT && threadIdx.x < BLK) s_qt[threadIdx.x] = qtable[threadIdx.x];
   if (lane == 0) { mbar_init(mb, 1); fence_mbar_init(); }
 

@@ -1569,6 +1569,65 @@ template <typename T> __device__ __forceinline__ T mul_rn(T a, T b);
 template <> __device__ __forceinline__ double mul_rn<double>(double a, double b) { return __dmul_rn(a, b); }
 template <> __device__ __forceinline__ float mul_rn<float>(float a, float b) { return __fmul_rn(a, b); }
 
+// The coefficients of a full block, already multiplied by sf (dctz-decomp-lib.c:392-416; the de-scale of :494-511 is folded
+// in).  Every decoder of full blocks -- the tile loops (decompress_tiles) and the range kernel (ranges.cuh) -- forms them
+// through these three, so that a block decodes to the same bits whichever way it is reached.
+// Bin centre of id (gen_bins / gen_bins_f, binning.c:19-22, 39-42).  Entry 255 is a dummy that an outlier replaces.
+template <typename T> __device__ __forceinline__ T center_coefficient(unsigned id, T bin_width, T sf) {
+  return mul_rn<T>(mul_rn<T>((T)center_multiple(id), bin_width), sf);
+}
+// Outlier `a` of AC_exact at coefficient position j, q = qtable[j] (only read in QT mode, :402-409 / :450-454).
+template <typename T, bool QT> __device__ __forceinline__ T outlier_coefficient(float a, T q, const QtConsts<T> &qk, T sf) {
+  T v;
+  if (QT) v = qt_unscale_one(a, q, qk); else v = (T)a;
+  return mul_rn<T>(v, sf);
+}
+template <typename T> __device__ __forceinline__ T dc_coefficient(float dc, T sf) { return mul_rn<T>((T)dc, sf); }  // :392
+
+// The partial last block (rem < 64 elements): coefficients by the definition, in double, through generic_idct; element n
+// (n < rem) is handed to store(n, value) by lane n % 32.  `base` = offset of the block's first outlier; a marker at or
+// past n_limit is a corrupt stream: the coefficient is 0 and on_corrupt() is called.  Used by k_tail_decompress and by
+// the range kernel.
+template <typename T, bool QT, class OnCorrupt, class Store>
+__device__ __forceinline__ void tail_block_decode(const uint8_t *__restrict__ bins, const float *__restrict__ dc_in, const float *__restrict__ ac_in,
+                                                  const T *__restrict__ qtable, int rem, unsigned long long blk_index, T bin_width, T sf,
+                                                  const QtConsts<T> &qk, unsigned long long base, unsigned long long n_limit,
+                                                  const OnCorrupt &on_corrupt, const Store &store, double *cs /* shared, BLK */, int lane) {
+  for (int h = 0; h < 2; h++) {
+    const int j = lane + 32 * h;
+    const bool valid = j < rem;
+    const unsigned id = valid ? bins[blk_index * BLK + j] : 0u;
+    const bool outl = valid && j > 0 && id == 255u;
+    const unsigned m = __ballot_sync(0xFFFFFFFFu, outl);
+    if (valid) {
+      T v;
+      if (j == 0) v = (T)dc_in[blk_index];
+      else if (outl) {
+        const unsigned long long at = base + __popc(m & ((1u << lane) - 1u));
+        float a = 0.f;
+        if (at < n_limit) a = ac_in[at]; else on_corrupt();  // more markers than outliers: corrupt stream
+        if (QT) v = (T)qt_unscale_one(a, qtable[j], qk); else v = (T)a;
+      } else {
+        if (sizeof(T) == 8) v = (T)__dmul_rn((double)center_multiple(id), (double)bin_width);
+        else v = (T)__fmul_rn((float)center_multiple(id), (float)bin_width);
+      }
+      cs[j] = (double)v;
+    }
+    base += __popc(m);
+  }
+  __syncwarp();
+  double r2[2];
+  generic_idct(cs, rem, lane, r2);
+  for (int h = 0; h < 2; h++) {
+    const int n = lane + 32 * h;
+    if (n < rem) {
+      T v = (T)r2[h];
+      if (sf != (T)1) v = v * sf;
+      store(n, v);
+    }
+  }
+}
+
 // Outlier extent of a tile (warp-uniform): where its run starts in AC_exact and how long it is.  The loads (load) and
 // the warp reduction that consumes them (finish) are a whole iteration apart, so their latency is never waited for.
 struct Extent { unsigned long long base; unsigned total; bool bad; };  // bad: the run would leave the caller's AC_exact array
@@ -1966,20 +2025,12 @@ __device__ __forceinline__ void decompress_tiles(const uint8_t *__restrict__ bin
 #pragma unroll
           for (int k = 0; k < 4; k++) {
             const unsigned i = i0 + 32 * k + lane;
-            if (i < ext_cur.total) {
-              T v;
-              if (QT) v = qt_unscale_one(a[k], s_qt[jpos[i]], qk); else v = (T)a[k];  // :402-409
-              dst[i] = mul_rn<T>(v, sf);                                               // and the de-scale
-            }
+            if (i < ext_cur.total) dst[i] = outlier_coefficient<T, QT>(a[k], QT ? s_qt[jpos[i]] : (T)0, qk, sf);
           }
         }
       } else {
         float *f = stage + pl.lead;
-        for (unsigned i = lane; i < ext_cur.total; i += 32) {
-          float v = f[i];
-          if (QT) v = (float)qt_unscale_one(v, s_qt[jpos[i]], qk);  // :450-454
-          f[i] = __fmul_rn(v, (float)sf);
-        }
+        for (unsigned i = lane; i < ext_cur.total; i += 32) f[i] = outlier_coefficient<T, QT>(f[i], QT ? s_qt[jpos[i]] : (T)0, qk, sf);
         rdy = reinterpret_cast<const T *>(f);
       }
       fence_async_smem();  // the stage was written through the generic proxy; TMA writes it next
@@ -1989,7 +2040,7 @@ __device__ __forceinline__ void decompress_tiles(const uint8_t *__restrict__ bin
 
     // ---- rebuild coefficients (dctz-decomp-lib.c:392-416), already multiplied by sf ----
     T x[BLK];
-    x[0] = mul_rn<T>((T)dcv, sf);  // :392
+    x[0] = dc_coefficient<T>(dcv, sf);
     if (ready && ext_cur.total != 0) {
       // marker 255 -> next finished outlier of this block, anything else -> its bin centre: one load either way
       const unsigned center_s = smem_u32(center);
@@ -2022,11 +2073,7 @@ __device__ __forceinline__ void decompress_tiles(const uint8_t *__restrict__ bin
           for (int b = 0; b < 8; b++) {
             const int j = 8 * g + b;
             const bool hit = ((b < 4 ? m0 >> (8 * b) : m1 >> (8 * (b - 4))) & 1u) != 0u;
-            if (hit) {
-              T v;
-              if (QT) v = qt_unscale_one(a[b], s_qt[j], qk); else v = (T)a[b];
-              x[j] = mul_rn<T>(v, sf);
-            }
+            if (hit) x[j] = outlier_coefficient<T, QT>(a[b], QT ? s_qt[j] : (T)0, qk, sf);
           }
         }
       }
@@ -2116,7 +2163,7 @@ k_decompress(const uint8_t *__restrict__ bins, const float *__restrict__ dc_in, 
   // bin centres: gen_bins / gen_bins_f (binning.c:19-22, 39-42): centre = (int multiple) * bin_width.  The de-scale
   // (x * sf, dctz-decomp-lib.c:494-511) is folded into the coefficients -- the inverse transform is linear, the
   // result moves by ~1 ulp -- so the table holds centre * sf.
-  for (int i = threadIdx.x; i < 256; i += Cfg::THREADS) center[i] = mul_rn<T>(mul_rn<T>((T)center_multiple((unsigned)i), bin_width), sf);
+  for (int i = threadIdx.x; i < 256; i += Cfg::THREADS) center[i] = center_coefficient<T>((unsigned)i, bin_width, sf);
   if (QT && threadIdx.x < BLK) s_qt[threadIdx.x] = qtable[threadIdx.x];
   if (lane == 0) { mbar_init(mb, 1); fence_mbar_init(); }
   __syncthreads();  // the only CTA-wide barrier before the epilogue
@@ -2179,40 +2226,9 @@ __global__ void __launch_bounds__(32) k_tail_decompress(const uint8_t *__restric
                                                         unsigned *corrupt_flag) {
   __shared__ double cs[BLK];
   const int lane = threadIdx.x;
-  unsigned long long base = n_consumed ? *n_consumed : pos0_if_no_full_blocks;
-  for (int h = 0; h < 2; h++) {
-    const int j = lane + 32 * h;
-    const bool valid = j < rem;
-    const unsigned id = valid ? bins[blk_index * BLK + j] : 0u;
-    const bool outl = valid && j > 0 && id == 255u;
-    const unsigned m = __ballot_sync(0xFFFFFFFFu, outl);
-    if (valid) {
-      T v;
-      if (j == 0) v = (T)dc_in[blk_index];
-      else if (outl) {
-        const unsigned long long at = base + __popc(m & ((1u << lane) - 1u));
-        float a = 0.f;
-        if (at < n_limit) a = ac_in[at]; else *corrupt_flag = 1u;  // more markers than outliers: corrupt stream
-        if (QT) v = (T)qt_unscale_one(a, qtable[j], qk); else v = (T)a;
-      } else {
-        if (sizeof(T) == 8) v = (T)__dmul_rn((double)center_multiple(id), (double)bin_width);
-        else v = (T)__fmul_rn((float)center_multiple(id), (float)bin_width);
-      }
-      cs[j] = (double)v;
-    }
-    base += __popc(m);
-  }
-  __syncwarp();
-  double r2[2];
-  generic_idct(cs, rem, lane, r2);
-  for (int h = 0; h < 2; h++) {
-    const int n = lane + 32 * h;
-    if (n < rem) {
-      T v = (T)r2[h];
-      if (sf != (T)1) v = v * sf;
-      out[blk_index * BLK + n] = v;
-    }
-  }
+  const unsigned long long base = n_consumed ? *n_consumed : pos0_if_no_full_blocks;
+  tail_block_decode<T, QT>(bins, dc_in, ac_in, qtable, rem, blk_index, bin_width, sf, qk, base, n_limit, [&] { *corrupt_flag = 1u; },
+                           [&](int n, T v) { out[blk_index * BLK + n] = v; }, cs, lane);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -227,6 +227,38 @@ int dctz_gpu_decompress_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bin_index, const
                             int datatype, double error_bound, double sf, int mode_qt, void *d_out,
                             uint32_t *d_corrupt, void *stream);
 
+/* ---- region decompression: element ranges of a slab without decoding the rest (DESIGN.md §4.4) ------------------
+ * The offset of a block's first outlier in AC_exact is the number of 255 markers in every block before it.  The outlier
+ * index holds that count per tile of 32 blocks, scanned, so that any block can be decoded on its own.  It is about
+ * 0.2 % of bin_index; its layout is private to the library.  A slab of a multi-GPU field gets its own index. */
+
+/* Bytes of the outlier index of an N-element slab (a function of N only). */
+size_t dctz_gpu_outlier_index_bytes(size_t N);
+
+/* Build the index of a slab's bin ids into the caller's device buffer d_index (16-byte aligned,
+ * outlier_index_bytes(N) bytes).  It is the same pre-pass decompress runs (k_count_bins + k_scan_groups),
+ * kept instead of discarded.  d_n_outliers (may be NULL): the number of outliers the bin ids mark
+ * (full blocks + tail), i.e. what a stream header's tot_AC_exact_count must say.  The index stays valid for as
+ * long as the bin ids do not change. */
+int dctz_gpu_outlier_index_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bin_index, size_t N, void *d_index,
+                               uint64_t *d_n_outliers, void *stream);
+
+/* Decode nranges element ranges of the slab.  d_ranges = nranges pairs {first element, count} (uint64, device).
+ * The ranges may come in any order and may overlap.  d_out receives their elements concatenated in range order
+ * (sum of counts elements; element-aligned).  Other arguments as in dctz_gpu_decompress_dev; the values are
+ * bit-identical to the same elements of dctz_gpu_decompress_dev's output.  d_index: built by
+ * dctz_gpu_outlier_index_dev for these bin ids and this N.
+ * *d_corrupt (may be NULL, cleared by the caller): bit 0 is set as in decompress_dev (more markers than outliers,
+ * or an index not built for this N: then nothing is written); bit 1 is set when a range leaves [0, N) or has
+ * count 0; that range's part of d_out (its stated count) is not written, the others are.  Bit 1 is also set, and nothing written, when the ranges touch more than
+ * 2^32 - 4096 tiles in all.  A range decodes every 64-element block it touches and reads the bin ids of its
+ * tile (2048 elements) from the tile's start: narrow ranges cost more per element than wide ones.          */
+int dctz_gpu_decompress_ranges_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bin_index, const float *d_DC,
+                                   const float *d_AC_exact, uint64_t n_outliers, const void *d_qtable, size_t N,
+                                   int datatype, double error_bound, double sf, int mode_qt, const void *d_index,
+                                   const uint64_t *d_ranges, size_t nranges, void *d_out, uint32_t *d_corrupt,
+                                   void *stream);
+
 /* x[i] <- x[i] / sf with IEEE division (the reference's in-place scaling, dctz-comp-lib.c:193-216),
  * and its inverse x[i] <- x[i] * sf (dctz-test.c:186-210, dctz-decomp-lib.c:494-511).          */
 int dctz_gpu_scale_dev(dctz_gpu_ctx *ctx, void *d_x, size_t N, int datatype, double sf, int multiply,
