@@ -298,15 +298,21 @@ static float threshold_f(int k) {
   return bits_to_f(hi);
 }
 
+// Compress admits max|x| in [T_{kmin-1}, T_kmax), i.e. sf = 10^(k-1) for k = kmin..kmax (DESIGN.md §2, "admitted exponent
+// range"): the kernels transform the UNSCALED block and quantise with kq = 1/(sf*bin_width), so below sf = 1e-302 (float
+// 1e-32) kq overflows at eb = 1E-6, and above sf = 1e305 (float 1e35) the unscaled transform overflows: the butterflies sum
+// all 64 values of a constant block before the factor 1/8, so 64 * max|x| must stay finite.
+// sfv holds one entry past the table (read, never used, by sf_window at the upper end).
+constexpr int SF_KMIN_D = -301, SF_KMAX_D = 306, SF_KMIN_F = -31, SF_KMAX_F = 36;
 static void build_sf_tables(dctz_gpu_ctx *c) {
-  const int kmin_d = -306, kmax_d = 308;  // sf = 10^(k-1) stays a normal double
+  const int kmin_d = SF_KMIN_D, kmax_d = SF_KMAX_D;
   c->min_d = threshold_d(kmin_d - 1);
   for (int k = kmin_d; k <= kmax_d; k++) {
     c->thr_d.push_back(threshold_d(k));
     c->sfv_d.push_back(pow(10, (double)k - 1));  // the literal expression of util.c:28 for ceil(.) == k
   }
   c->sfv_d.push_back(pow(10, (double)(kmax_d + 1) - 1));
-  const int kmin_f = -36, kmax_f = 38;
+  const int kmin_f = SF_KMIN_F, kmax_f = SF_KMAX_F;
   c->min_f = threshold_f(kmin_f - 1);
   for (int k = kmin_f; k <= kmax_f; k++) {
     c->thr_f.push_back(threshold_f(k));
@@ -426,10 +432,12 @@ static int ctx_init(dctz_gpu_ctx *ctx, int device) {
   TRY(upload_table(ctx, ctx->sfv_f, &ctx->tb.sf_f));
   ctx->tb.n_d = (int)ctx->thr_d.size();
   ctx->tb.n_f = (int)ctx->thr_f.size();
-  ctx->tb.kmin_d = -306;
-  ctx->tb.kmin_f = -36;
+  ctx->tb.kmin_d = SF_KMIN_D;
+  ctx->tb.kmin_f = SF_KMIN_F;
   ctx->tb.min_d = ctx->min_d;
   ctx->tb.min_f = ctx->min_f;
+  ctx->tb.max_d = ctx->thr_d.back();
+  ctx->tb.max_f = ctx->thr_f.back();
   // kernel attributes + residency (persistent grids are sized from these)
   ctx->occ[0][1][0] = kernel_occupancy(k_compress<double, false, false>, CompressCfg<double, false>::THREADS, CompressCfg<double, false>::SMEM);
   ctx->occ[0][1][1] = kernel_occupancy(k_compress<double, true, false>, CompressCfg<double, true>::THREADS, CompressCfg<double, true>::SMEM);
@@ -517,11 +525,11 @@ extern "C" void dctz_gpu_host_free(void *p) { if (p) cudaFreeHost(p); }
 extern "C" double dctz_gpu_sf_from_max(const dctz_gpu_ctx *ctx, double max_abs, int datatype) {
   if (!ctx) return 0.0;
   if (datatype == DCTZ_GPU_DOUBLE) {
-    if (!(max_abs >= ctx->min_d) || isinf(max_abs)) return 0.0;
+    if (!(max_abs >= ctx->min_d && max_abs < ctx->thr_d.back())) return 0.0;  // outside the admitted range (also NaN, inf)
     return ctx->sfv_d[host_lookup(ctx->thr_d, max_abs)];
   }
   const float m = (float)max_abs;
-  if (!(m >= ctx->min_f) || isinf(m)) return 0.0;
+  if (!(m >= ctx->min_f && m < ctx->thr_f.back())) return 0.0;
   return (double)ctx->sfv_f[host_lookup(ctx->thr_f, m)];
 }
 
@@ -1160,6 +1168,30 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
   return DCTZ_GPU_OK;
 }
 
+// sf comes from the stream header and may be any decade the reference writes (double 1e-307..1e308, float 1e-37..1e38).
+// The decoders form c*sf BEFORE the inverse transform: near the top a scaled DC of up to 80 times sf overflows, near the
+// bottom the coefficients become subnormal and lose bits.  Outside 2^-960..2^960 (float 2^-96..2^96) the kernels decode
+// with sf*2^-E instead (E = the binary exponent of sf: an exact rescaling that commutes with every step of the decode) and
+// k_scale multiplies the reconstruction by 2^E afterwards.  Returns E, or 0 inside the window (no extra pass).
+static int decode_exponent(double sf, int datatype) {
+  const bool dbl = datatype == DCTZ_GPU_DOUBLE;
+  const int e = dbl ? ilogb(sf) : ilogbf((float)sf);
+  const int w = dbl ? 960 : 96;
+  return (e > w || e < -w) ? e : 0;
+}
+static double decode_sf(double sf, int datatype, int E) {
+  return datatype == DCTZ_GPU_DOUBLE ? ldexp(sf, -E) : (double)ldexpf((float)sf, -E);
+}
+static int rescale_output(dctz_gpu_ctx *ctx, void *d_out, size_t N, int datatype, int E, cudaStream_t st) {
+  const size_t want = (N + 255) / 256;
+  const int grid = (int)(want < (size_t)ctx->sm_count * 16 ? want : (size_t)ctx->sm_count * 16);
+  if (datatype == DCTZ_GPU_DOUBLE) k_scale<double><<<grid, 256, 0, st>>>((double *)d_out, N, ldexp(1.0, E), 1);
+  else k_scale<float><<<grid, 256, 0, st>>>((float *)d_out, N, ldexpf(1.0f, E), 1);
+  ctx->launches++;
+  CU(cudaGetLastError());
+  return DCTZ_GPU_OK;
+}
+
 extern "C" int dctz_gpu_decompress_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const float *d_dc, const float *d_ac,
                                        uint64_t n_outliers, const void *d_qtable, size_t N, int datatype, double eb, double sf, int mode_qt,
                                        void *d_out, uint32_t *d_corrupt, void *stream) {
@@ -1172,12 +1204,16 @@ extern "C" int dctz_gpu_decompress_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bins,
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
   unsigned *flag = d_corrupt ? (unsigned *)d_corrupt : &ctx->d_ctl[1].corrupt;  // the caller's flag, else a scratch word nobody reads
+  const int E = decode_exponent(sf, datatype);
+  const double sfk = decode_sf(sf, datatype, E);
   if (datatype == DCTZ_GPU_DOUBLE) {
-    if (mode_qt) return launch_decompress<double, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sf, (double *)d_out, flag, st);
-    return launch_decompress<double, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sf, (double *)d_out, flag, st);
+    if (mode_qt) TRY((launch_decompress<double, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sfk, (double *)d_out, flag, st)));
+    else TRY((launch_decompress<double, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sfk, (double *)d_out, flag, st)));
+  } else {
+    if (mode_qt) TRY((launch_decompress<float, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sfk, (float *)d_out, flag, st)));
+    else TRY((launch_decompress<float, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sfk, (float *)d_out, flag, st)));
   }
-  if (mode_qt) return launch_decompress<float, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, (float *)d_out, flag, st);
-  return launch_decompress<float, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, (float *)d_out, flag, st);
+  return E ? rescale_output(ctx, d_out, N, datatype, E, st) : DCTZ_GPU_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1246,21 +1282,26 @@ extern "C" int dctz_gpu_outlier_index_dev(dctz_gpu_ctx *ctx, const uint8_t *d_bi
   return DCTZ_GPU_OK;
 }
 
+// The range plan in ctx->region: [RangeCtl (128 B)][piece_at, out_at: per range][chunk_piece, chunk_out: per chunk of 1024]
+static RangePlan range_plan_view(void *region, size_t nranges) {
+  char *p = (char *)region;
+  RangePlan plan;
+  plan.ctl = (RangeCtl *)p;
+  plan.piece_at = (unsigned long long *)(p + 128);
+  plan.out_at = plan.piece_at + nranges;
+  plan.chunk_piece = (unsigned long long *)(p + 128 + up128(nranges * 16));
+  plan.chunk_out = plan.chunk_piece + (nranges + 1023) / 1024;
+  return plan;
+}
+
 template <typename T, bool QT>
 static int launch_ranges(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const float *d_dc, const float *d_ac, unsigned long long n_outliers, const T *d_qtable,
                          size_t N, double eb, double sf, const void *d_index, const unsigned long long *d_ranges, size_t nranges, T *d_out,
                          unsigned *flag, cudaStream_t st) {
   typedef RangeCfg<T> Cfg;
   const size_t nchunks = (nranges + 1023) / 1024;
-  const size_t off_ranges = 128, off_chunks = off_ranges + up128(nranges * 16);
-  TRY(grow(ctx, ctx->region, off_chunks + up128(nchunks * 16), true));  // (a new allocation starts zeroed: RangeCtl::done)
-  char *p = (char *)ctx->region.p;
-  RangePlan plan;
-  plan.ctl = (RangeCtl *)p;
-  plan.piece_at = (unsigned long long *)(p + off_ranges);
-  plan.out_at = plan.piece_at + nranges;
-  plan.chunk_piece = (unsigned long long *)(p + off_chunks);
-  plan.chunk_out = plan.chunk_piece + nchunks;
+  TRY(grow(ctx, ctx->region, 128 + up128(nranges * 16) + up128(nchunks * 16), true));  // (a new allocation starts zeroed: RangeCtl::done)
+  const RangePlan plan = range_plan_view(ctx->region.p, nranges);
   const RegionIndex idx = region_view(d_index, N);
   k_range_plan<<<(unsigned)nchunks, 1024, 0, st>>>(d_ranges, nranges, N, idx.hdr, plan, flag);
   ctx->launches++;
@@ -1298,12 +1339,24 @@ extern "C" int dctz_gpu_decompress_ranges_dev(dctz_gpu_ctx *ctx, const uint8_t *
   cudaStream_t st = (cudaStream_t)stream;
   unsigned *flag = d_corrupt ? (unsigned *)d_corrupt : &ctx->d_ctl[1].corrupt;  // the caller's flag, else a scratch word nobody reads
   const unsigned long long *rg = (const unsigned long long *)d_ranges;
+  const int E = decode_exponent(sf, datatype);
+  const double sfk = decode_sf(sf, datatype, E);
   if (datatype == DCTZ_GPU_DOUBLE) {
-    if (mode_qt) return launch_ranges<double, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sf, d_index, rg, nranges, (double *)d_out, flag, st);
-    return launch_ranges<double, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sf, d_index, rg, nranges, (double *)d_out, flag, st);
+    if (mode_qt) TRY((launch_ranges<double, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sfk, d_index, rg, nranges, (double *)d_out, flag, st)));
+    else TRY((launch_ranges<double, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const double *)d_qtable, N, eb, sfk, d_index, rg, nranges, (double *)d_out, flag, st)));
+  } else {
+    if (mode_qt) TRY((launch_ranges<float, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sfk, d_index, rg, nranges, (float *)d_out, flag, st)));
+    else TRY((launch_ranges<float, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sfk, d_index, rg, nranges, (float *)d_out, flag, st)));
   }
-  if (mode_qt) return launch_ranges<float, true>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, d_index, rg, nranges, (float *)d_out, flag, st);
-  return launch_ranges<float, false>(ctx, d_bins, d_dc, d_ac, n_outliers, (const float *)d_qtable, N, eb, sf, d_index, rg, nranges, (float *)d_out, flag, st);
+  if (!E) return DCTZ_GPU_OK;
+  // the plan launch_ranges left in ctx->region: output offsets per range (the decode wrote the places of the valid ranges)
+  const RangePlan plan = range_plan_view(ctx->region.p, nranges);
+  const int grid = ctx->sm_count * 8;
+  if (datatype == DCTZ_GPU_DOUBLE) k_scale_ranges<double><<<grid, 256, 0, st>>>((double *)d_out, rg, nranges, N, plan, ldexp(1.0, E));
+  else k_scale_ranges<float><<<grid, 256, 0, st>>>((float *)d_out, rg, nranges, N, plan, ldexpf(1.0f, E));
+  ctx->launches++;
+  CU(cudaGetLastError());
+  return DCTZ_GPU_OK;
 }
 
 extern "C" int dctz_gpu_scale_dev(dctz_gpu_ctx *ctx, void *d_x, size_t N, int datatype, double sf, int multiply, void *stream) {

@@ -47,8 +47,8 @@ template <> struct QuantConsts<float> {
 };
 
 struct SfTables {         // host libm results, see build_sf_tables() in dctz_gpu.cu
-  const double *thr_d; const double *sf_d; int n_d, kmin_d; double min_d;  // thr[i] = T_{kmin+i}; valid for max|x| >= min_d
-  const float *thr_f; const float *sf_f; int n_f, kmin_f; float min_f;
+  const double *thr_d; const double *sf_d; int n_d, kmin_d; double min_d, max_d;  // thr[i] = T_{kmin+i}; admitted: min_d <= max|x| < max_d
+  const float *thr_f; const float *sf_f; int n_f, kmin_f; float min_f, max_f;
   int qmax_words;          // 64-bit words of the QT per-position maxima to clear (64 elements of T)
 };
 
@@ -81,6 +81,10 @@ __device__ __forceinline__ void finalize_params(const double *stats_all, int nra
                                                 int is_double, double first_value, int first_slab,
                                                 const SfTables &tb, DevParams *p, Info *info,
                                                 unsigned long long *qmax_zero);
+
+// max(a, b) that returns a NaN operand (fmax drops it): merges of partial maxima must keep a NaN of the data visible to
+// finalize_params, which rejects it
+__device__ __forceinline__ double max_keep_nan(double a, double b) { return (a > b || a != a) ? a : b; }
 
 template <typename T>
 __global__ void __launch_bounds__(256) k_stats(const T *__restrict__ in, size_t n, StatPartial *partials,
@@ -267,15 +271,17 @@ __device__ __forceinline__ void finalize_params(const double *stats_all, int nra
   if (qmax_zero) for (int j = 0; j < tb.qmax_words; j++) qmax_zero[j] = 0ull;  // QT per-position maxima
   double mx = stats_all[0], mn = stats_all[1], sum = stats_all[2];
   for (int r = 1; r < nranks; r++) {  // rank order => deterministic sum
-    mx = fmax(mx, stats_all[3 * r]);
+    mx = max_keep_nan(mx, stats_all[3 * r]);
     mn = fmin(mn, stats_all[3 * r + 1]);
     sum += stats_all[3 * r + 2];
   }
   if (first_slab) sum -= first_value;  // util.c:21-25: the running sum starts at element 1
+  // DCTZ_GPU_EDEGENERATE: max|x| is 0, inf or NaN (every statistics pass keeps a NaN in the maximum), or outside the admitted
+  // range (build_sf_tables).  The sum of finite data may overflow (the reference's sum and mean become inf as well; the
+  // decoder never reads the mean): it is not a test for non-finite data.
   int status = 0;
-  if (!(mx > 0.0) || !(mx < __longlong_as_double(0x7FF0000000000000ll))) status = -5;  // DCTZ_GPU_EDEGENERATE
   double sf = 1.0, mean;
-  if (!status && (is_double ? !(mx >= tb.min_d) : !((float)mx >= tb.min_f))) status = -5;  // sf would be subnormal
+  if (is_double ? !(mx >= tb.min_d && mx < tb.max_d) : !((float)mx >= tb.min_f && (float)mx < tb.max_f)) status = -5;
   p->decade_lo = 0.0;
   p->decade_hi = __longlong_as_double(0x7FF0000000000000ll);
   if (is_double) {
@@ -304,7 +310,6 @@ __device__ __forceinline__ void finalize_params(const double *stats_all, int nra
     p->sf_d = sf; p->inv_sf_d = 0.0;
   }
   if (!(sf > 0.0)) status = -5;
-  if (!(sum - sum == 0.0)) status = -5;  // a NaN or an infinity among the data (the single-read path takes max|x| with FP max, which skips NaN)
   p->status = status;
   info->sf = sf; info->mean = mean; info->max_abs = mx; info->min_abs = mn; info->sum = sum;
   info->n_outliers = 0; info->n_edge = 0; info->n_exact_path = 0; info->n_qt_dropped = 0;
@@ -568,6 +573,13 @@ __device__ __forceinline__ double fmax_t(double a, double b) { return fmax(a, b)
 __device__ __forceinline__ float fmax_t(float a, float b) { return fmaxf(a, b); }
 __device__ __forceinline__ double fmin_t(double a, double b) { return fmin(a, b); }
 __device__ __forceinline__ float fmin_t(float a, float b) { return fminf(a, b); }
+
+// Out of line: the path of a refused field only, kept out of the register allocation of the compress kernels' tile loop.
+__device__ __noinline__ void zero_tile_counts(unsigned *counts, unsigned long long nblk_full) {
+  const unsigned long long ntiles = (nblk_full + WTILE - 1) / WTILE;
+  for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < ntiles; i += (unsigned long long)gridDim.x * blockDim.x)
+    counts[i] = 0u;
+}
 
 // VERIFY: what a thread has seen of the slab's true statistics while compressing with a BELIEF about them.
 template <typename T> struct VerifyStat {
@@ -852,6 +864,13 @@ k_compress(const __grid_constant__ CUtensorMap tmap_in, unsigned long long nblk_
     if (src.first_slab) fv = src.is_double ? __ldg((const double *)src.first_elem) : (double)__ldg((const float *)src.first_elem);
     finalize_params(src.stats_all, src.nranks, src.n_total, src.is_double, fv, src.first_slab, src.tb, &s_params, &s_info,
                     (blockIdx.x == 0 && src.mode != MODE_REDO) ? src.qmax_zero : nullptr);
+    if (VERIFY && s_params.status != 0) {
+      // A refused BELIEF (0, NaN, inf, or outside the admitted exponent range -- a caller's bound may be DBL_MAX) must not
+      // skip the tile loop: the loop is what gathers the true statistics the REDO launch decides on.  Compress with the
+      // placeholder belief max|x| = 1 instead; the REDO launch recompresses (or refuses) from the true statistics.
+      const double one[3] = {1.0, 1.0, 0.0};
+      finalize_params(one, 1, src.n_total, src.is_double, 0.0, 0, src.tb, &s_params, &s_info, nullptr);
+    }
     int skip = 0;
     if (src.mode == MODE_REDO) {
       skip = (s_params.status == 0 && s_params.sf_d == *reinterpret_cast<volatile double *>(&ctl->belief_sf)) ? 1 : 0;
@@ -866,7 +885,12 @@ k_compress(const __grid_constant__ CUtensorMap tmap_in, unsigned long long nblk_
     }
   }
   __syncthreads();  // the only CTA-wide barrier before the epilogue
-  if (s_skip) return;
+  if (s_skip) {
+    // degenerate statistics: no tile is compressed, so no tile writes its outlier count -- zero them all, or the scan and
+    // gather launched after this kernel would move stale or uninitialised counts' worth of outliers
+    if (s_params.status != 0) zero_tile_counts(counts, nblk_full);
+    return;
+  }
 
   VerifyStat<T> vstat;
   vstat.tile_sums = src.tile_sums;
@@ -949,7 +973,7 @@ __global__ void __launch_bounds__(256) k_reduce_tiles(const double *__restrict__
   true3[2] = t;
   if (sizeof(T) == 4) {  // float: the "high word" is the whole pattern -- exact
     double mx = (double)__int_as_float((int)x), mn = (double)__int_as_float((int)n);
-    if (tail3) { mx = fmax(mx, tail3[0]); mn = fmin(mn, tail3[1]); }
+    if (tail3) { mx = max_keep_nan(mx, tail3[0]); mn = fmin(mn, tail3[1]); }
     true3[0] = mx; true3[1] = mn;
   } else {
     r.hw[0] = x; r.hw[1] = n;
@@ -1019,7 +1043,7 @@ __global__ void __launch_bounds__(256) k_resolve_extremes(const double *__restri
   __threadfence();
   double mx = __longlong_as_double((long long)*reinterpret_cast<volatile unsigned long long *>(r.ext_bits));
   double mn = __longlong_as_double((long long)*reinterpret_cast<volatile unsigned long long *>(r.ext_bits + 1));
-  if (tail3) { mx = fmax(mx, tail3[0]); mn = fmin(mn, tail3[1]); }
+  if (tail3) { mx = max_keep_nan(mx, tail3[0]); mn = fmin(mn, tail3[1]); }
   true3[0] = mx; true3[1] = mn;
   *done2 = 0u;
 }
@@ -1063,7 +1087,7 @@ __global__ void __launch_bounds__(256) k_sample(const T *__restrict__ in, size_t
   double tmax = 0.0, tmin = inf, tsum = 0.0;
   for (size_t k = nfull; k < n; k++) {  // the partial tail block, exactly
     const double v = (double)in[k], a = fabs(v);
-    tmax = fmax(tmax, a); tmin = fmin(tmin, a); tsum += v;
+    tmax = max_keep_nan(tmax, a); tmin = fmin(tmin, a); tsum += v;  // (a NaN stays in the maximum: finalize_params rejects it)
   }
   tail3[0] = tmax; tail3[1] = tmin; tail3[2] = tsum;
   mx = fmax(mx, tmax);
@@ -1128,7 +1152,10 @@ __global__ void __launch_bounds__(32) k_tail_compress(const T *__restrict__ in /
                                                       T *qtable0, Info *info) {
   __shared__ double xs[BLK];
   const int lane = threadIdx.x;
-  if (params->status != 0) return;  // degenerate statistics: nothing is compressed
+  if (params->status != 0) {  // degenerate statistics: nothing is compressed; the scan and gather that follow see no outliers
+    if (lane == 0) counts[slot_tile] = 0u;
+    return;
+  }
   const T sf = (sizeof(T) == 8) ? (T)params->sf_d : (T)params->sf_f;
   for (int n = lane; n < rem; n += 32) {
     T v = in[n];

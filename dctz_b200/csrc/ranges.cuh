@@ -111,6 +111,25 @@ __global__ void __launch_bounds__(1024) k_range_plan(const unsigned long long *_
   }
 }
 
+// out *= s over the places of the ranges k_decompress_ranges wrote (those inside [0, n)): the second half of a decode with
+// a rescaled sf (dctz_gpu.cu: decode_exponent).  The places of skipped ranges stay untouched.  Fewer ranges than CTAs (a
+// few long ranges, e.g. one whole field): the whole grid strides over each range in turn; else one CTA per range.
+template <typename T>
+__global__ void __launch_bounds__(256) k_scale_ranges(T *__restrict__ out, const unsigned long long *__restrict__ ranges, unsigned long long nranges,
+                                                      unsigned long long n, RangePlan plan, T s) {
+  if (__ldg(&plan.ctl->pieces) == 0ull) return;  // the decode kernel wrote nothing
+  const bool whole_grid = nranges < gridDim.x;
+  const unsigned long long first = whole_grid ? 0ull : blockIdx.x, step = whole_grid ? 1ull : gridDim.x;
+  const unsigned long long t0 = whole_grid ? (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x : threadIdx.x;
+  const unsigned long long ts = whole_grid ? (unsigned long long)gridDim.x * blockDim.x : blockDim.x;
+  for (unsigned long long r = first; r < nranges; r += step) {
+    const unsigned long long a = __ldg(ranges + 2 * r), c = __ldg(ranges + 2 * r + 1);
+    if (c == 0 || a >= n || c > n - a) continue;
+    T *dst = out + __ldg(plan.out_at + r) + __ldg(plan.chunk_out + (r >> 10));
+    for (unsigned long long i = t0; i < c; i += ts) dst[i] = dst[i] * s;
+  }
+}
+
 template <typename T> struct RangeCfg {
   static constexpr int WARPS = 4;
   static constexpr int THREADS = WARPS * 32;

@@ -49,7 +49,8 @@ extern "C" {
 #define DCTZ_GPU_ECUDA (-2)     /* a CUDA call failed */
 #define DCTZ_GPU_EINVAL (-3)    /* bad argument (eb < 1e-6 like dctz-comp-lib.c:135, alignment, ...) */
 #define DCTZ_GPU_ENOMEM (-4)
-#define DCTZ_GPU_EDEGENERATE (-5) /* max|x| is 0, inf or NaN: the reference computes sf = 0/NaN (util.c:28) */
+#define DCTZ_GPU_EDEGENERATE (-5) /* max|x| is 0, inf or NaN (the reference computes sf = 0/NaN, util.c:28), or outside
+                                     the exponent range compress admits (sf 1e-302..1e305, float 1e-32..1e35: DESIGN.md §2) */
 #define DCTZ_GPU_ESTALE (-6)      /* (no longer returned: a wrong belief about the statistics is corrected on the device) */
 #define DCTZ_GPU_ECORRUPT (-7)    /* decompress_core: bin_index marks more outliers than AC_exact holds */
 

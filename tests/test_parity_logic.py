@@ -107,3 +107,83 @@ def test_wrong_outlier_value_fails():
     g["ac"][7] = np.float32(g["ac"][7] * (1 + 1e-5))
     with pytest.raises(AssertionError, match="outlier values differ"):
         parity.compare_compress(g, orc, x, 1e-3, False, ctx=FakeCtx())
+
+
+class FakeDecoder:
+    """stands in for dctz_b200.Context.decompress_core: the oracle's own reconstruction, optionally perturbed"""
+
+    def __init__(self, perturb=None):
+        self.perturb = perturb
+
+    def decompress_core(self, bins, dc, ac, n, dtype, eb, sf, qt=False, qtable=None):
+        r = reflib.oracle_decompress(bins, dc, ac, qtable, n, eb, sf, qt, dtype)
+        return self.perturb(r, sf) if self.perturb else r
+
+
+def _tiny_field():
+    """double field at the bottom of the exponent range (sf = 1e-307): one block of small values among larger ones"""
+    t = np.arange(64 * 40, dtype=np.float64)
+    x = 3.0 + np.sin(t / 29.0) * 2.0
+    x[64 * 7:64 * 8] = 1e-3 * np.cos(t[:64] / 5.0)
+    return x * 1e-307
+
+
+def test_decompress_tolerance_has_no_absolute_floor_and_follows_the_block():
+    x = _tiny_field()
+    parity.check_decompress(FakeDecoder(), x, 1e-3, False)  # the oracle against itself
+
+    def shift_all(r, sf):  # 1e-9 of sf everywhere: 1e3 times the tolerance, but far below the old 1e-300 floor
+        return r + 1e-9 * sf
+
+    with pytest.raises(AssertionError, match="beyond the tolerance"):
+        parity.check_decompress(FakeDecoder(shift_all), x, 1e-3, False)
+
+    def shift_small_block(r, sf):  # within RTOL of the FIELD's maximum, far outside RTOL of block 7's
+        r = r.copy()
+        r[64 * 7 + 3] += 1e-12 * sf
+        return r
+
+    with pytest.raises(AssertionError, match="beyond the tolerance"):
+        parity.check_decompress(FakeDecoder(shift_small_block), x, 1e-3, False)
+
+    def make_inf(r, sf):
+        r = r.copy()
+        r[5] = np.inf
+        return r
+
+    with pytest.raises(AssertionError, match="non-finite"):
+        parity.check_decompress(FakeDecoder(make_inf), x, 1e-3, False)
+
+
+def test_equal_infinite_sums_agree_and_a_finite_sum_never_matches_an_infinite_one():
+    x = np.full(1 << 16, 3e304)  # sum 1.97e309
+    orc = reflib.oracle_compress(x, 1e-3, False)
+    assert orc["stat"]["sum"] == np.inf  # the reference's running sum overflows
+    g = _fake_gpu(orc)
+    parity.compare_compress(g, orc, x, 1e-3, False, ctx=FakeCtx())
+    g["info"]["sum"] = 1.7e308
+    with pytest.raises(AssertionError):
+        parity.compare_compress(g, orc, x, 1e-3, False, ctx=FakeCtx())
+    g["info"]["sum"] = -np.inf
+    with pytest.raises(AssertionError):
+        parity.compare_compress(g, orc, x, 1e-3, False, ctx=FakeCtx())
+    assert parity.sums_agree(np.inf, np.inf, x, 1e304) and not parity.sums_agree(np.inf, 1e308, x, 1e304)
+    assert not parity.sums_agree(1e308, np.inf, x, 1e304)
+
+
+class OverflowCtx(FakeCtx):
+    """a transform that overflowed: every coefficient infinite"""
+
+    def dct_blocks(self, x, dn=64, inverse=False):
+        return np.full_like(x, np.inf)
+
+
+def test_a_non_finite_gpu_coefficient_is_a_failure_not_a_tie():
+    x, eb = _field(np.float64, 3e-4)
+    orc = reflib.oracle_compress(x, eb, False)
+    g = _fake_gpu(orc)
+    j = 1
+    t = parity.ordinal_of(g["bin_index"][j:j + 1], orc["coef"][j:j + 1])[0]
+    g["bin_index"][j] = 254 - 2 * (t - 1) if t - 1 <= 127 else 2 * (t - 1 - 127) - 1  # the bin below
+    with pytest.raises(AssertionError, match="non-finite"):
+        parity.compare_compress(g, orc, x, eb, False, ctx=OverflowCtx())
