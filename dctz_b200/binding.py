@@ -24,7 +24,7 @@ EXPORTS = [
     "dctz_gpu_sf_from_max", "dctz_gpu_selftest_division", "dctz_gpu_launch_count", "dctz_gpu_compress_core_cb",
     "dctz_gpu_set_timing", "dctz_gpu_last_call_stats", "dctz_gpu_fused_phase_times", "dctz_gpu_compress_slab_comm",
     "dctz_gpu_sample_dev", "dctz_gpu_compress_spec_dev", "dctz_gpu_compress_spec_finish_dev",
-    "dctz_gpu_outlier_index_bytes", "dctz_gpu_outlier_index_dev", "dctz_gpu_decompress_ranges_dev",
+    "dctz_gpu_outlier_index_bytes", "dctz_gpu_outlier_index_dev", "dctz_gpu_decompress_ranges_dev", "dctz_gpu_launch_plan",
 ]
 
 
@@ -44,6 +44,16 @@ class GpuInfo(C.Structure):  # dctz_gpu_info
 
 
 INFO_BYTES = C.sizeof(GpuInfo)
+
+
+class LaunchPlan(C.Structure):  # dctz_gpu_plan
+    _fields_ = [(k, C.c_uint64) for k in (
+        "fused_compress_grid", "fused_decompress_grid", "ntiles", "n_entries", "compress_grid", "compress_warps", "compress_batch",
+        "reduce_ctas", "scan_chunks", "groups", "gather_grid", "qt_max_groups", "qt_max_grid", "decompress_grid", "decompress_batch",
+        "decompress_scan_chunks", "ahead_grid", "ahead_batch", "ahead_units", "ahead_groups", "ahead_super")]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
 _lib = None
 
 
@@ -90,6 +100,7 @@ def load_library():
         "dctz_gpu_sf_from_max": (dbl, [vp, dbl, i32]),
         "dctz_gpu_selftest_division": (i32, [vp, i32, dbl, u64, C.c_uint32, C.POINTER(u64)]),
         "dctz_gpu_launch_count": (u64, [vp]),
+        "dctz_gpu_launch_plan": (i32, [vp, sz, i32, i32, C.POINTER(LaunchPlan)]),
         "dctz_gpu_compress_core_cb": (i32, [vp, vp, sz, i32, dbl, i32, vp, vp, vp, vp, vp, vp, C.POINTER(GpuInfo), vp, vp]),
         "dctz_gpu_set_timing": (i32, [vp, i32]),
         "dctz_gpu_fused_phase_times": (i32, [vp, i32, C.POINTER(dbl)]),
@@ -184,6 +195,13 @@ class Context:
     @property
     def launch_count(self):
         return int(self._lib.dctz_gpu_launch_count(self._h))
+
+    def launch_plan(self, n, dtype, qt=False):
+        """the grids, tiles per ticket and scratch partitions this context's kernels would run with for a slab of n
+        elements (dctz_gpu_plan, as a dict); launches nothing"""
+        p = LaunchPlan()
+        self._check(self._lib.dctz_gpu_launch_plan(self._h, int(n), _code(dtype), int(bool(qt)), C.byref(p)))
+        return p.as_dict()
 
     def set_timing(self, on):
         return self._lib.dctz_gpu_set_timing(self._h, int(bool(on)))

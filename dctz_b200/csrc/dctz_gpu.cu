@@ -585,11 +585,76 @@ static bool aligned16(const void *p) { return ((uintptr_t)p & 15u) == 0; }
 static unsigned tile_batch(size_t ntiles, size_t nwarps, bool compress = false) {
   return ntiles >= 16 * nwarps ? (compress ? DCTZ_TILE_BATCH_C : DCTZ_TILE_BATCH_D) : 1u;
 }
+static size_t scan_chunks(size_t n_entries) { return ((n_entries + 31) / 32 + 1023) / 1024; }  // k_scan_groups CTAs
+
+// Single-launch path (fused.cuh): whole fields of full blocks up to fused_max_bytes, all CTAs co-resident.
+static int fused_grid(const dctz_gpu_ctx *ctx, int kernel, size_t N, size_t es, int mode_qt) {
+  static const bool dbg = getenv("DCTZ_DEBUG") != nullptr;
+  if (dbg)
+    fprintf(stderr, "fused_grid: kernel %d N %zu es %zu qt %d coop %d max_bytes %zu occ %d\n", kernel, N, es, mode_qt, ctx->coop, ctx->fused_max_bytes,
+            ctx->occ_fused[kernel][es == 8][mode_qt ? 1 : 0]);
+  if (!ctx->coop || N % BLK || N == 0 || N * es > ctx->fused_max_bytes) return 0;
+  const size_t ntiles = (N / BLK + WTILE - 1) / WTILE;
+  const size_t resident = (size_t)ctx->sm_count * ctx->occ_fused[kernel][es == 8][mode_qt ? 1 : 0];
+  if (resident == 0) return 0;
+  const size_t grid = ntiles < resident ? ntiles : resident;
+  if ((ntiles + grid - 1) / grid > FUSED_MAX_TILES_PER_CTA) return 0;
+  return (int)grid;
+}
+
+// The launch plan of a slab of N elements (dctz_gpu_plan): the streaming launches below take their grids, tiles per
+// ticket and scratch partitions from here, and dctz_gpu_launch_plan reports the same values.
+static_assert(CompressCfg<double, false>::WARPS == 4 && CompressCfg<double, true>::WARPS == 4 && CompressCfg<float, false>::WARPS == 4 &&
+              CompressCfg<float, true>::WARPS == 4 && DecompressCfg<double, false>::WARPS == 4 && DecompressCfg<double, true>::WARPS == 4 &&
+              DecompressCfg<float, false>::WARPS == 4 && DecompressCfg<float, true>::WARPS == 4, "make_plan assumes 4 warps per CTA");
+constexpr size_t PLAN_WARPS = 4;
+static size_t clamp_grid(size_t want, size_t cap) { return want < cap ? want : cap; }
+static size_t gather_grid(const dctz_gpu_ctx *ctx, size_t n_entries) {  // one CTA per group of 32 entries, at most 8 per SM
+  const size_t groups = (n_entries + 31) / 32;
+  return clamp_grid(groups ? groups : 1, (size_t)ctx->sm_count * 8);
+}
+static dctz_gpu_plan make_plan(const dctz_gpu_ctx *ctx, size_t N, size_t es, int mode_qt) {
+  dctz_gpu_plan p = {};
+  const int dbl = es == 8, qt = mode_qt ? 1 : 0;
+  const size_t sm = (size_t)ctx->sm_count;
+  p.fused_compress_grid = (uint64_t)fused_grid(ctx, 0, N, es, qt);
+  p.fused_decompress_grid = (uint64_t)fused_grid(ctx, 1, N, es, qt);
+  const size_t ntiles = (N / BLK + WTILE - 1) / WTILE, ctas = (ntiles + PLAN_WARPS - 1) / PLAN_WARPS;
+  p.ntiles = ntiles;
+  p.n_entries = ntiles + (N % BLK ? 1 : 0);  // the partial tail block is one more "tile" of the compress scratch
+  p.compress_grid = clamp_grid(ctas, sm * ctx->occ[0][dbl][qt]);
+  p.compress_warps = p.compress_grid * PLAN_WARPS;
+  p.compress_batch = tile_batch(ntiles, p.compress_warps, true);
+  p.reduce_ctas = (ntiles + 4095) / 4096;
+  p.groups = (p.n_entries + 31) / 32;
+  p.scan_chunks = scan_chunks(p.n_entries);
+  p.gather_grid = gather_grid(ctx, p.n_entries);
+  p.qt_max_groups = (ntiles + 31) / 32;
+  p.qt_max_grid = clamp_grid(p.qt_max_groups, sm * 8);
+  p.decompress_grid = clamp_grid(ctas, sm * ctx->occ[1][dbl][qt]);
+  p.decompress_batch = tile_batch(ntiles, p.decompress_grid * PLAN_WARPS);
+  p.decompress_scan_chunks = scan_chunks(ntiles);
+  p.ahead_grid = clamp_grid(ctas, sm * ctx->occ_ahead[dbl][qt]);
+  p.ahead_batch = tile_batch(ntiles, p.ahead_grid * PLAN_WARPS);
+  p.ahead_units = (ntiles + p.ahead_batch - 1) / p.ahead_batch;
+  p.ahead_groups = (p.ahead_units + 63) / 64;
+  p.ahead_super = (p.ahead_units + 2047) / 2048;
+  return p;
+}
+
+extern "C" int dctz_gpu_launch_plan(const dctz_gpu_ctx *ctx, size_t N, int datatype, int mode_qt, dctz_gpu_plan *out) {
+  if (!ctx) return fail(nullptr, DCTZ_GPU_EINVAL, "ctx is NULL");
+  dctz_gpu_ctx *c = const_cast<dctz_gpu_ctx *>(ctx);  // (for the error message only)
+  if (datatype != DCTZ_GPU_FLOAT && datatype != DCTZ_GPU_DOUBLE) return fail(c, DCTZ_GPU_EINVAL, "datatype %d is neither FLOAT(0) nor DOUBLE(1)", datatype);
+  if (!out || N == 0) return fail(c, DCTZ_GPU_EINVAL, "launch_plan: NULL pointer or N == 0");
+  *out = make_plan(ctx, N, datatype == DCTZ_GPU_DOUBLE ? 8 : 4, mode_qt);
+  return DCTZ_GPU_OK;
+}
 
 struct ScanBufs { unsigned *counts; ScanOut out; unsigned nchunks; };
 static size_t up128(size_t v) { return (v + 127) / 128 * 128; }
 static int scan_bufs(dctz_gpu_ctx *ctx, size_t n_entries, ScanBufs *sb) {
-  const size_t ngroups = (n_entries + 31) / 32, nchunks = (ngroups + 1023) / 1024;
+  const size_t ngroups = (n_entries + 31) / 32, nchunks = scan_chunks(n_entries);
   TRY(grow(ctx, ctx->status, up128(ngroups * 8) + up128(nchunks * 8) + up128(n_entries * 4)));
   char *p = (char *)ctx->status.p;
   sb->out.group_prefix = (unsigned long long *)p;
@@ -683,8 +748,9 @@ static int launch_compress(dctz_gpu_ctx *ctx, const T *d_in, size_t N, double eb
   const unsigned long long nblk_full = N / BLK;
   const int rem = (int)(N % BLK);
   const QuantConsts<T> qc = make_quant<T>(eb);
-  const size_t ntiles = (nblk_full + WTILE - 1) / WTILE;
-  const size_t n_entries = ntiles + (rem ? 1 : 0);  // the partial tail block is one more "tile" of the scratch layout
+  const dctz_gpu_plan plan = make_plan(ctx, N, sizeof(T), QT);
+  const size_t ntiles = plan.ntiles;
+  const size_t n_entries = plan.n_entries;  // the partial tail block is one more "tile" of the scratch layout
   if (n_entries > 0xFFFFF000ull) return fail(ctx, DCTZ_GPU_EINVAL, "slab too large: %zu tiles", n_entries);
   ScanBufs sb;
   TRY(scan_bufs(ctx, n_entries, &sb));
@@ -711,23 +777,21 @@ static int launch_compress(dctz_gpu_ctx *ctx, const T *d_in, size_t N, double eb
   src.params = ctx->d_params;
   src.qmax_zero = QT ? (unsigned long long *)d_qtable_raw : nullptr;
   src.tile_sums = nullptr; src.tile_ext = nullptr;
-  const size_t nred = (ntiles + 4095) / 4096;  // CTAs of k_reduce_tiles
+  const size_t nred = plan.reduce_ctas;  // CTAs of k_reduce_tiles
   if (sa.mode == MODE_BELIEF) {  // scratch: [tile sums][CTA sums][tile extremes][CTA extremes]
     TRY(grow(ctx, ctx->tile_sums, (ntiles + nred + 8) * sizeof(double) + (ntiles + nred + 8) * sizeof(uint2)));
     src.tile_sums = (double *)ctx->tile_sums.p;
     src.tile_ext = (uint2 *)((double *)ctx->tile_sums.p + ntiles + nred + 8);
   }
   if (nblk_full) {
-    const size_t resident = (size_t)ctx->sm_count * ctx->occ[0][sizeof(T) == 8][QT];
-    const size_t ctas = (ntiles + Cfg::WARPS - 1) / Cfg::WARPS;
-    const int grid = (int)(ctas < resident ? ctas : resident);
+    const int grid = (int)plan.compress_grid;
     CUtensorMap tmap;
     TRY(make_tile_map(ctx, &tmap, d_in, BLK * sizeof(T), nblk_full));
     fused.out = sb.out;
     fused.total = &d_info->n_outliers;
     // small field, true statistics: the last CTA scans (one launch less); the single-read modes scan after the REDO launch
-    fused.n_entries = (sa.mode == MODE_STATS && rem == 0 && (n_entries + 31) / 32 <= 1024) ? (unsigned)n_entries : 0u;
-    const unsigned batch = tile_batch(ntiles, (size_t)grid * Cfg::WARPS, true);
+    fused.n_entries = (sa.mode == MODE_STATS && rem == 0 && plan.groups <= 1024) ? (unsigned)n_entries : 0u;
+    const unsigned batch = (unsigned)plan.compress_batch;
     if (sa.mode == MODE_BELIEF)
       k_compress<T, QT, true><<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(tmap, nblk_full, src, qc, d_bins, d_dc, sb.counts, ac_slots, raw, jpos,
                                                                      (T *)d_qtable_raw, &ctx->d_ctl[0], d_info, fused, batch);
@@ -757,8 +821,7 @@ static int launch_compress(dctz_gpu_ctx *ctx, const T *d_in, size_t N, double eb
     }
     if (QT) {  // per-position maxima of the parked (unscaled) outliers, scaled by the kernel's last CTA (before the tail
                // block adds its own, scaled, values)
-      const size_t groups = (ntiles + 31) / 32;
-      const int gq = (int)(groups < (size_t)ctx->sm_count * 8 ? groups : (size_t)ctx->sm_count * 8);
+      const int gq = (int)plan.qt_max_grid;
       k_qt_max<T><<<gq, 256, 0, st>>>(sb.counts, (unsigned)ntiles, raw, jpos, (U *)d_qtable_raw, ctx->d_params, ctx->d_done + 4);
       ctx->launches++;
     }
@@ -779,8 +842,7 @@ static int launch_compress(dctz_gpu_ctx *ctx, const T *d_in, size_t N, double eb
     ctx->launches++;
   }
   if (!QT) {
-    const size_t want = (n_entries + 31) / 32;  // one CTA per group of 32 tiles
-    const int grid = (int)(want < (size_t)ctx->sm_count * 8 ? want : (size_t)ctx->sm_count * 8);
+    const int grid = (int)plan.gather_grid;  // one CTA per group of 32 tiles
     k_gather_ec<<<grid, 256, 0, st>>>(sb.counts, sb.out.group_prefix, sb.out.chunk_prefix, (unsigned)n_entries, ac_slots, d_ac, &d_info->n_outliers);
     ctx->launches++;
   }
@@ -887,8 +949,7 @@ static int launch_qt_finish(dctz_gpu_ctx *ctx, double eb, const T *d_qraw, T *d_
   const unsigned n_entries = ctx->qt_entries;
   ScanBufs sb;
   TRY(scan_bufs(ctx, n_entries, &sb));  // same layout as in the compress call: nothing is reallocated
-  const size_t want = ((size_t)n_entries + 31) / 32;  // one CTA per group of 32 tiles
-  const int grid = (int)(want < (size_t)ctx->sm_count * 8 ? (want ? want : 1) : (size_t)ctx->sm_count * 8);
+  const int grid = (int)gather_grid(ctx, n_entries);  // as planned for the compress call
   k_qt_gather<T><<<grid, 256, 0, st>>>(sb.counts, sb.out.group_prefix, sb.out.chunk_prefix, n_entries, (const T *)qt_raw_slots(ctx), (const uint8_t *)qt_j_slots(ctx),
                                        d_qraw, d_qtable, k, d_ac, d_info, ctx->d_params, ctx->qt_tail_tile);
   ctx->launches++;
@@ -906,21 +967,6 @@ extern "C" int dctz_gpu_qt_finish_dev(dctz_gpu_ctx *ctx, int datatype, double eb
   if (datatype == DCTZ_GPU_DOUBLE)
     return launch_qt_finish<double>(ctx, eb, (const double *)d_qtable_raw, (double *)d_qtable, d_ac, (Info *)d_info, st);
   return launch_qt_finish<float>(ctx, eb, (const float *)d_qtable_raw, (float *)d_qtable, d_ac, (Info *)d_info, st);
-}
-
-// Single-launch path (fused.cuh): whole fields of full blocks up to fused_max_bytes, all CTAs co-resident.
-static int fused_grid(const dctz_gpu_ctx *ctx, int kernel, size_t N, size_t es, int mode_qt) {
-  static const bool dbg = getenv("DCTZ_DEBUG") != nullptr;
-  if (dbg)
-    fprintf(stderr, "fused_grid: kernel %d N %zu es %zu qt %d coop %d max_bytes %zu occ %d\n", kernel, N, es, mode_qt, ctx->coop, ctx->fused_max_bytes,
-            ctx->occ_fused[kernel][es == 8][mode_qt ? 1 : 0]);
-  if (!ctx->coop || N % BLK || N == 0 || N * es > ctx->fused_max_bytes) return 0;
-  const size_t ntiles = (N / BLK + WTILE - 1) / WTILE;
-  const size_t resident = (size_t)ctx->sm_count * ctx->occ_fused[kernel][es == 8][mode_qt ? 1 : 0];
-  if (resident == 0) return 0;
-  const size_t grid = ntiles < resident ? ntiles : resident;
-  if ((ntiles + grid - 1) / grid > FUSED_MAX_TILES_PER_CTA) return 0;
-  return (int)grid;
 }
 
 template <typename T, bool QT>
@@ -1081,9 +1127,10 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
   // gen_bins: bin_width = error_bound*2*BRSF (binning.c:16); gen_bins_f receives the bound as float (binning.c:32-36)
   const T bw = (sizeof(T) == 8) ? (T)(eb * 2 * 1.0) : (T)(float)((float)eb * 2 * 1.0);
   const T sfT = (T)sf;
-  if (const int fgrid = fused_grid(ctx, 1, N, sizeof(T), QT)) {  // small field of full blocks: count + dequantise + IDCT in ONE launch
+  const dctz_gpu_plan plan = make_plan(ctx, N, sizeof(T), QT);
+  if (const int fgrid = (int)plan.fused_decompress_grid) {  // small field of full blocks: count + dequantise + IDCT in ONE launch
     unsigned long long nb = nblk_full;
-    const size_t ntiles = (nblk_full + WTILE - 1) / WTILE;
+    const size_t ntiles = plan.ntiles;
     ScanBufs sb;
     TRY(scan_bufs(ctx, ntiles, &sb));
     TRY(grow(ctx, ctx->tile_off, ntiles * sizeof(unsigned)));
@@ -1104,7 +1151,7 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
     return DCTZ_GPU_OK;
   }
   if (nblk_full) {
-    const size_t ntiles = (nblk_full + WTILE - 1) / WTILE;
+    const size_t ntiles = plan.ntiles;
     if (ntiles > 0xFFFFF000ull) return fail(ctx, DCTZ_GPU_EINVAL, "slab too large: %zu tiles", ntiles);
     // No pre-pass (the warps count ahead and look their offsets up, AheadExtents) where it pays: the count-ahead kernel saves
     // the second read of the bin ids and costs ~15 % more instructions -- measured 1.68 against 1.71 ms on the outlier-free 8 GiB
@@ -1112,11 +1159,9 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
     // number of outliers, so the choice is made per call: below one outlier per 128 elements.
     const bool ahead = ctx->decomp_ahead > 0 || (ctx->decomp_ahead < 0 && ac_limit <= (unsigned long long)(N >> 7));
     if (ahead) {
-      const size_t resident = (size_t)ctx->sm_count * ctx->occ_ahead[sizeof(T) == 8][QT];
-      const size_t ctas = (ntiles + Cfg::WARPS - 1) / Cfg::WARPS;
-      const int grid = (int)(ctas < resident ? ctas : resident);
-      const unsigned batch = tile_batch(ntiles, (size_t)grid * Cfg::WARPS);
-      const size_t nunits = (ntiles + batch - 1) / batch, ngroups = (nunits + 63) / 64, nsuper = (nunits + 2047) / 2048;
+      const int grid = (int)plan.ahead_grid;
+      const unsigned batch = (unsigned)plan.ahead_batch;
+      const size_t nunits = plan.ahead_units, ngroups = plan.ahead_groups, nsuper = plan.ahead_super;
       const size_t off_s = up128(nunits * sizeof(unsigned)), off_t = off_s + up128(ngroups * 8), total = off_t + up128(nsuper * 8);
       TRY(grow(ctx, ctx->ahead_buf, total));
       CU(cudaMemsetAsync(ctx->ahead_buf.p, 0, total, st));
@@ -1146,15 +1191,13 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
         ctx->launches++;
       }
     }
-    const size_t resident = (size_t)ctx->sm_count * ctx->occ[1][sizeof(T) == 8][QT];
-    const size_t ctas = (ntiles + Cfg::WARPS - 1) / Cfg::WARPS;
-    const int grid = (int)(ctas < resident ? ctas : resident);
+    const int grid = (int)plan.decompress_grid;
     CUtensorMap tmap;
     TRY(make_tile_map(ctx, &tmap, d_out, BLK * sizeof(T), nblk_full));
     k_decompress<T, QT, false><<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(d_bins, d_dc, d_ac, d_qtable, nblk_full, bw, sfT, qk, tmap, sb.counts,
                                                                       sb.out.group_prefix, sb.out.chunk_prefix, ctx->d_nconsumed, ac_limit,
                                                                       &ctx->d_ctl[1], d_corrupt, aligned16(d_dc) ? 1 : 0,
-                                                                      tile_batch(ntiles, (size_t)grid * Cfg::WARPS), ctx->l2_hints > 0 ? ctx->l2_hints : 0);
+                                                                      (unsigned)plan.decompress_batch, ctx->l2_hints > 0 ? ctx->l2_hints : 0);
     ctx->launches++;
     CU(cudaGetLastError());
     }

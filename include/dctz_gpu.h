@@ -295,6 +295,28 @@ int dctz_gpu_selftest_division(dctz_gpu_ctx *ctx, int datatype, double b, uint64
                                uint64_t *mismatches);
 /* Number of kernels launched by this context so far (bench.py's gpu_launches).                  */
 uint64_t dctz_gpu_launch_count(const dctz_gpu_ctx *ctx);
+
+/* Launch plan of a slab of N elements: the grids, tiles per ticket and scratch partitions the kernels of this
+ * context would be launched with (they depend on the SM count and on the kernels' measured residency).  The
+ * launch code takes these values from the same helper, so a caller -- a test that must reach a regime, a
+ * benchmark that reports one -- sees exactly what runs.  Host-only, launches nothing.  A tile is 32 blocks
+ * (2048 elements); a group is 32 tiles; a scan chunk is 1024 groups; "entries" are the tiles plus one for a
+ * partial tail block.  The streaming values are filled in even where the single-launch kernels would run.    */
+typedef struct dctz_gpu_plan {
+  uint64_t fused_compress_grid;   /* compress_field_dev / compress_core: CTAs of the single-launch kernel, 0 = streaming */
+  uint64_t fused_decompress_grid; /* decompress_dev: the same for the single-launch decoder                              */
+  uint64_t ntiles, n_entries;
+  uint64_t compress_grid, compress_warps, compress_batch; /* k_compress: CTAs, warps, tiles per ticket               */
+  uint64_t reduce_ctas;           /* k_reduce_tiles (single-read path): one CTA per 4096 tiles                         */
+  uint64_t scan_chunks;           /* k_scan_groups CTAs over the compress entries                                      */
+  uint64_t groups;                /* groups of 32 entries (compress)                                                   */
+  uint64_t gather_grid;           /* k_gather_ec / k_qt_gather CTAs over `groups`                                      */
+  uint64_t qt_max_groups, qt_max_grid; /* k_qt_max: groups of 32 tiles, CTAs                                           */
+  uint64_t decompress_grid, decompress_batch, decompress_scan_chunks; /* k_decompress after the pre-pass             */
+  uint64_t ahead_grid, ahead_batch, ahead_units, ahead_groups, ahead_super; /* count-ahead k_decompress: units of
+                                                                     `ahead_batch` tiles, groups of 64 units, super-groups of 2048 */
+} dctz_gpu_plan;
+int dctz_gpu_launch_plan(const dctz_gpu_ctx *ctx, size_t N, int datatype, int mode_qt, dctz_gpu_plan *out);
 /* Stage timers of the host-buffer calls (the reference prints sf_t / dct_t / idct_t under -DTIME_DEBUG,
  * dctz-comp-lib.c:762-773, dctz-decomp-lib.c:513-528).  set_timing(1) makes compress_core / decompress_core run
  * upload, statistics and transform strictly one after the other with CUDA events between them (the default

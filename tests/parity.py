@@ -135,7 +135,16 @@ def sums_agree(got, want, x, sf):
             return np.sign(got) == np.sign(want) and abs(got) > float(np.finfo(np.float32).max)
         return got == want
     rel = 1e-9 if np.dtype(x.dtype) == np.float64 else 2e-3
-    return abs(got / sf - want / sf) <= rel * float(np.sum(np.abs(x.astype(np.float64) / sf)))
+    if abs(got / sf - want / sf) <= rel * float(np.sum(np.abs(x.astype(np.float64) / sf))):
+        return True
+    if np.dtype(x.dtype) != np.float32:
+        return False
+    # The reference adds float data into a float, one element after the other (util.c:35-40): its error grows with n, up
+    # to (n - 2) * 2^-24 * sum|x| (recursive summation), and past ~2^24 elements it can stall far from the sum.  The GPU's
+    # double sum must then agree with the exact sum of x[1..n-1] instead, and the reference's lie within its own bound.
+    xs = x[1:].astype(np.float64)
+    exact, mag = float(np.sum(xs)), float(np.sum(np.abs(xs)))  # pairwise: ~log2(n) * 2^-53 * mag from the exact value
+    return abs(got - exact) <= 1e-9 * mag and abs(want - exact) <= max(x.size - 2, 1) * 2.0 ** -24 * mag * 1.01
 
 
 def decode_tolerance(want, sf):

@@ -55,6 +55,20 @@ def test_info_struct_layout():
     assert binding.INFO_BYTES == 80  # 5 doubles + 4 u64 + 2 i32, mirrored by a static_assert in dctz_gpu.cu
 
 
+def test_plan_struct_mirrors_the_header():
+    """binding.LaunchPlan lists the fields of dctz_gpu_plan in the header's order (all uint64_t)"""
+    txt = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "dctz_gpu.h")).read(), flags=re.S)
+    body = re.search(r"typedef struct dctz_gpu_plan \{(.*?)\} dctz_gpu_plan;", txt, flags=re.S).group(1)
+    fields = []
+    for decl in body.split(";"):
+        decl = decl.strip()
+        if decl:
+            assert decl.startswith("uint64_t "), decl
+            fields += [f.strip() for f in decl[len("uint64_t "):].split(",")]
+    assert fields == [k for k, _ in binding.LaunchPlan._fields_]
+    assert C.sizeof(binding.LaunchPlan) == 8 * len(fields)
+
+
 def test_product_does_not_touch_the_oracle():
     """nothing under dctz_b200/ or include/ may import, link or call oracle/ (it is test infrastructure)."""
     bad = []

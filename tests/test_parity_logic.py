@@ -187,3 +187,17 @@ def test_a_non_finite_gpu_coefficient_is_a_failure_not_a_tie():
     g["bin_index"][j] = 254 - 2 * (t - 1) if t - 1 <= 127 else 2 * (t - 1 - 127) - 1  # the bin below
     with pytest.raises(AssertionError, match="non-finite"):
         parity.compare_compress(g, orc, x, eb, False, ctx=OverflowCtx())
+
+
+def test_a_float_sum_the_reference_could_not_accumulate():
+    """2^25 floats near 25: the reference's float running sum stalls near 2^29 (each addend is below half an ulp), so the
+    GPU's double sum is judged against the exact sum instead -- and a wrong GPU sum still fails"""
+    x = (25.0 + np.sin(np.arange(1 << 25) / 77.0)).astype(np.float32)
+    ref = reflib.oracle_stat(x)
+    exact = float(np.sum(x[1:].astype(np.float64)))
+    assert abs(ref["sum"] - exact) > 0.1 * exact  # the reference's own sum is far off
+    assert parity.sums_agree(exact, ref["sum"], x, ref["sf"])
+    assert not parity.sums_agree(exact * (1 + 1e-6), ref["sum"], x, ref["sf"])
+    assert not parity.sums_agree(ref["sum"] * 1.5, ref["sum"], x, ref["sf"])
+    # double data keeps the tight rule alone
+    assert not parity.sums_agree(exact, ref["sum"], x.astype(np.float64), ref["sf"])
