@@ -279,7 +279,7 @@ struct TileControl {
   unsigned done;     // CTAs that have exited; the last one resets the fields for the next launch
   unsigned long long max_bits;  // VERIFY variant of K2: largest |x| bit pattern seen so far
   unsigned corrupt;  // K3: set when the bin indices mark more outliers than the caller's AC_exact array holds
-  unsigned pad_;
+  unsigned count_ticket;  // K3 without the pre-pass: next unit to count
   unsigned long long min_bits;  // VERIFY: smallest |x| bit pattern (kept at ~0 between launches)
   double belief_sf;             // the scaling factor the VERIFY launch compressed with (read by the REDO launch)
 };

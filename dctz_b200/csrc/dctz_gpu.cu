@@ -204,9 +204,9 @@ struct dctz_gpu_ctx {
   double *d_dfrag2[2] = {nullptr, nullptr}; // ... of its even / odd halves (k_dct64_dmma_split)
   int occ[2][2][2] = {};  // resident CTAs/SM per [kernel][datatype][qt]
   int occ_ahead[2][2] = {};  // ... of the count-ahead decompress kernel [datatype][qt]
-  int decomp_ahead = -1;     // DCTZ_DECOMP_AHEAD: 1 = streaming decompress always without the pre-pass, 0 = never, unset = where the stated outlier density is below 1/128 (DESIGN.md 4.3)
+  int decomp_ahead = -1;     // DCTZ_DECOMP_AHEAD: 1 = streaming decompress always without the pre-pass, 0 = never, unset = double where the stated outlier density is below 1/128, float never (DESIGN.md 4.3)
   int l2_hints = -1;         // DCTZ_L2_HINTS: bit 0 stores evict_first, bit 1 bin-id copies evict_first, bit 2 pre-pass path: tiles from the last one down; -1 = 3 for the count-ahead path, 0 otherwise
-  DevBuf ahead_buf;          // count-ahead decompress: agg[u] | S[u/64] | T[u/2048], zeroed before every launch
+  DevBuf ahead_buf;          // decompress without the pre-pass: counts[t] | agg[u] | S[u/64] | T[u/2048], zeroed before every launch
   // single-launch kernels for small fields (fused.cuh)
   int occ_fused[2][2][2] = {};
   size_t fused_max_bytes = (size_t)256 << 20;  // fields up to this size take the single-launch path (DCTZ_FUSED_MAX_MB, 0 = never)
@@ -360,6 +360,14 @@ extern "C" void dctz_gpu_destroy(dctz_gpu_ctx *ctx) {
   for (double *p : ctx->d_dfrag2) if (p) cudaFree(p);
   if (ctx->chunk_stats.p) cudaFree(ctx->chunk_stats.p);
   if (ctx->ahead_buf.p) cudaFree(ctx->ahead_buf.p);
+#ifdef DCTZ_WAIT_STATS
+  {
+    unsigned long long w[3] = {};
+    if (cudaMemcpyFromSymbol(w, g_wait_stats, sizeof w) == cudaSuccess)
+      fprintf(stderr, "dctz wait stats: %llu units counted, decode re-reads of unpublished counts %llu, count-warp looks at a closed lead window %llu\n",
+              w[2], w[0], w[1]);
+  }
+#endif
   delete ctx->pool;
   for (int i = 0; i < NSTAGE; i++) {
     if (ctx->stage[i]) cudaFreeHost(ctx->stage[i]);
@@ -453,10 +461,10 @@ static int ctx_init(dctz_gpu_ctx *ctx, int device) {
   ctx->occ[1][1][1] = kernel_occupancy(k_decompress<double, true, false>, DecompressCfg<double, true>::THREADS, DecompressCfg<double, true>::SMEM);
   ctx->occ[1][0][0] = kernel_occupancy(k_decompress<float, false, false>, DecompressCfg<float, false>::THREADS, DecompressCfg<float, false>::SMEM);
   ctx->occ[1][0][1] = kernel_occupancy(k_decompress<float, true, false>, DecompressCfg<float, true>::THREADS, DecompressCfg<float, true>::SMEM);
-  ctx->occ_ahead[1][0] = kernel_occupancy(k_decompress<double, false, true>, DecompressCfg<double, false>::THREADS, DecompressCfg<double, false>::SMEM);
-  ctx->occ_ahead[1][1] = kernel_occupancy(k_decompress<double, true, true>, DecompressCfg<double, true>::THREADS, DecompressCfg<double, true>::SMEM);
-  ctx->occ_ahead[0][0] = kernel_occupancy(k_decompress<float, false, true>, DecompressCfg<float, false>::THREADS, DecompressCfg<float, false>::SMEM);
-  ctx->occ_ahead[0][1] = kernel_occupancy(k_decompress<float, true, true>, DecompressCfg<float, true>::THREADS, DecompressCfg<float, true>::SMEM);
+  ctx->occ_ahead[1][0] = kernel_occupancy(k_decompress<double, false, true>, SplitCfg::THREADS, DecompressCfg<double, false>::SMEM);
+  ctx->occ_ahead[1][1] = kernel_occupancy(k_decompress<double, true, true>, SplitCfg::THREADS, DecompressCfg<double, true>::SMEM);
+  ctx->occ_ahead[0][0] = kernel_occupancy(k_decompress<float, false, true>, SplitCfg::THREADS, DecompressCfg<float, false>::SMEM);
+  ctx->occ_ahead[0][1] = kernel_occupancy(k_decompress<float, true, true>, SplitCfg::THREADS, DecompressCfg<float, true>::SMEM);
   {
     const char *e = getenv("DCTZ_DECOMP_AHEAD");
     ctx->decomp_ahead = e ? atoi(e) : -1;  // -1: by the outlier density of the call
@@ -582,6 +590,7 @@ static bool aligned16(const void *p) { return ((uintptr_t)p & 15u) == 0; }
 #ifndef DCTZ_TILE_BATCH_D
 #define DCTZ_TILE_BATCH_D 4u
 #endif
+static_assert(DCTZ_TILE_BATCH_D <= 32, "CountedExtents holds the counts of a unit's tiles in the lanes of a warp");
 static unsigned tile_batch(size_t ntiles, size_t nwarps, bool compress = false) {
   return ntiles >= 16 * nwarps ? (compress ? DCTZ_TILE_BATCH_C : DCTZ_TILE_BATCH_D) : 1u;
 }
@@ -1153,25 +1162,28 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
   if (nblk_full) {
     const size_t ntiles = plan.ntiles;
     if (ntiles > 0xFFFFF000ull) return fail(ctx, DCTZ_GPU_EINVAL, "slab too large: %zu tiles", ntiles);
-    // No pre-pass (the warps count ahead and look their offsets up, AheadExtents) where it pays: the count-ahead kernel saves
-    // the second read of the bin ids and costs ~15 % more instructions -- measured 1.68 against 1.71 ms on the outlier-free 8 GiB
-    // slab, 0.53 against 0.51 ms with 5 % outliers, whose tile loop has no issue slots to spare.  The caller states the
-    // number of outliers, so the choice is made per call: below one outlier per 128 elements.
-    const bool ahead = ctx->decomp_ahead > 0 || (ctx->decomp_ahead < 0 && ac_limit <= (unsigned long long)(N >> 7));
+    // No pre-pass (a count warpgroup publishes the tiles' outlier counts beside the decode warpgroup, count_units) where it
+    // pays, DESIGN.md 4.3.  double: below one outlier per 128 elements (the caller states the number of outliers, so the
+    // choice is made per call): 1.57 against 1.69 ms on the outlier-free 8 GiB slab, but 0.539 against 0.505 ms with 5 %
+    // outliers (B200).  float: never -- the pre-pass kernel keeps 3 CTAs of decode warps per SM, the split kernel fits 2
+    // (f32 slab 1.037 against 1.129 ms).
+    const bool ahead = ctx->decomp_ahead > 0 || (ctx->decomp_ahead < 0 && sizeof(T) == 8 && ac_limit <= (unsigned long long)(N >> 7));
     if (ahead) {
       const int grid = (int)plan.ahead_grid;
       const unsigned batch = (unsigned)plan.ahead_batch;
       const size_t nunits = plan.ahead_units, ngroups = plan.ahead_groups, nsuper = plan.ahead_super;
-      const size_t off_s = up128(nunits * sizeof(unsigned)), off_t = off_s + up128(ngroups * 8), total = off_t + up128(nsuper * 8);
+      const size_t off_a = up128(ntiles * sizeof(unsigned)), off_s = off_a + up128(nunits * sizeof(unsigned)), off_t = off_s + up128(ngroups * 8),
+                   total = off_t + up128(nsuper * 8);
       TRY(grow(ctx, ctx->ahead_buf, total));
       CU(cudaMemsetAsync(ctx->ahead_buf.p, 0, total, st));
-      unsigned *agg = (unsigned *)ctx->ahead_buf.p;
-      unsigned long long *S = (unsigned long long *)((char *)ctx->ahead_buf.p + off_s), *Tt = (unsigned long long *)((char *)ctx->ahead_buf.p + off_t);
+      char *ab = (char *)ctx->ahead_buf.p;
+      unsigned *tile_counts = (unsigned *)ab, *agg = (unsigned *)(ab + off_a);
+      unsigned long long *S = (unsigned long long *)(ab + off_s), *Tt = (unsigned long long *)(ab + off_t);
       CUtensorMap tmap;
       TRY(make_tile_map(ctx, &tmap, d_out, BLK * sizeof(T), nblk_full));
-      k_decompress<T, QT, true><<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(d_bins, d_dc, d_ac, d_qtable, nblk_full, bw, sfT, qk, tmap, agg, S, Tt,
-                                                                       ctx->d_nconsumed, ac_limit, &ctx->d_ctl[1], d_corrupt, aligned16(d_dc) ? 1 : 0,
-                                                                       batch, ctx->l2_hints < 0 ? 3 : ctx->l2_hints);
+      k_decompress<T, QT, true><<<grid, SplitCfg::THREADS, Cfg::SMEM, st>>>(d_bins, d_dc, d_ac, d_qtable, nblk_full, bw, sfT, qk, tmap, tile_counts, agg,
+                                                                            S, Tt, ctx->d_nconsumed, ac_limit, &ctx->d_ctl[1], d_corrupt,
+                                                                            aligned16(d_dc) ? 1 : 0, batch, ctx->l2_hints < 0 ? 3 : ctx->l2_hints);
       ctx->launches++;
       CU(cudaGetLastError());
     } else {
@@ -1194,7 +1206,7 @@ static int launch_decompress(dctz_gpu_ctx *ctx, const uint8_t *d_bins, const flo
     const int grid = (int)plan.decompress_grid;
     CUtensorMap tmap;
     TRY(make_tile_map(ctx, &tmap, d_out, BLK * sizeof(T), nblk_full));
-    k_decompress<T, QT, false><<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(d_bins, d_dc, d_ac, d_qtable, nblk_full, bw, sfT, qk, tmap, sb.counts,
+    k_decompress<T, QT, false><<<grid, Cfg::THREADS, Cfg::SMEM, st>>>(d_bins, d_dc, d_ac, d_qtable, nblk_full, bw, sfT, qk, tmap, sb.counts, nullptr,
                                                                       sb.out.group_prefix, sb.out.chunk_prefix, ctx->d_nconsumed, ac_limit,
                                                                       &ctx->d_ctl[1], d_corrupt, aligned16(d_dc) ? 1 : 0,
                                                                       (unsigned)plan.decompress_batch, ctx->l2_hints > 0 ? ctx->l2_hints : 0);

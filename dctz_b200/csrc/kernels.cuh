@@ -1695,22 +1695,56 @@ struct ScannedExtents {
 };
 
 // ------------------------------------------------------------------------------------------
-// Decompress WITHOUT the pre-pass (k_count_bins + k_scan_groups): every warp counts the markers of the tiles it is going to
-// process AHEAD tiles before it processes them -- 64 bytes of bin ids per lane, loaded at the top of an iteration and
-// counted at its end, with the evict_last hint so that the lines are still in L2 when the tile's bulk copy asks for them --
-// and PUBLISHES the count of every finished unit (a ticket's batch of tiles) in three levels:
-//     agg[u]      the unit's outliers                                   (flag bit 31 | count)
-//     S[u / 64]   sum over the group of 64 units, by atomic addition    (contributions << 48 | sum)
-//     T[u / 2048] sum over the super-group of 32 groups, likewise       (contributions << 48 | sum)
-// The offset of a unit's first outlier is then a pure READ: complete super-groups below it + complete groups of its
-// super-group below it + the units of its group below it -- five coalesced loads, no chain of waiting warps: nobody
-// waits for a prefix, only (and by then never in practice: the counts were published AHEAD tiles ago) for counts, and
-// counting never waits for anything.  Units are handed out in increasing order, so every unit below a ticketed one has an
-// owner that is resident and publishes it before it waits for anything itself: no deadlock.
-// The object is both the tile sequence (advance) and the extent source (load / finish) of decompress_tiles.
+// Decompress WITHOUT the pre-pass (k_count_bins + k_scan_groups), warp-specialised: k_decompress<T, QT, true> runs two
+// warpgroups per CTA.
+//   count  (warps 4-7): take units (a ticket's batch of tiles) in increasing order from a count ticket of their own, load
+//          the units' bin ids with the evict_last hint (the decode warps' bulk copies then find them in L2), count the
+//          markers and PUBLISH them:
+//              counts[t]   the tile's outliers                                   (flag bit 31 | count)
+//              agg[u]      the unit's outliers                                   (flag bit 31 | count)
+//              S[u / 64]   sum over the group of 64 units, by atomic addition    (contributions << 48 | sum)
+//              T[u / 2048] sum over the super-group of 32 groups, likewise       (contributions << 48 | sum)
+//          Every entry carries its own completion mark on a buffer the host zeroes before the launch, so a publish needs no
+//          fence and a reader no acquire: a value is either marked complete or read again.
+//   decode (warps 0-3): the tile loop of the pre-pass kernel (decompress_tiles) over units from the decode ticket, with the
+//          extents of CountedExtents: a unit's first outlier is a pure READ (complete super-groups below it + complete
+//          groups of its super-group below it + the units of its group below it -- five coalesced loads), a tile's is that
+//          plus the counts of the earlier tiles of its unit, and both are loaded one iteration before they are used.
+// The counting thereby leaves the decode warps' dependent chain, and setmaxnreg hands the registers the count warps do not
+// need (COUNT_REGS) to the decode warps (DECODE_REGS).
+// Deadlock freedom.  Counters wait only for the decode TICKET (unit u is counted once u < decode tickets taken + COUNT_LEAD),
+// never for a decode to complete; decoders wait only for counts.  Both tickets are taken only by running warps, in
+// increasing order.  Let D be the number of decode tickets taken.  A decoder waits only for units below its own, i.e. below
+// D.  A counter holding a unit below D + COUNT_LEAD never waits; a counter that waits holds a unit >= D + COUNT_LEAD, so
+// the count ticket has passed every unit below D, and each of those belongs to a running counter that does not wait: every
+// unit below D is published, no decoder waits for ever, and D grows until it passes the last unit, which releases every
+// counter.  A CTA that is not resident holds no ticket of either kind, so two such kernels of two contexts sharing the
+// device (neither fully resident) cannot wait for each other's missing CTAs.
 // ------------------------------------------------------------------------------------------
-struct AheadBufs { unsigned *agg; unsigned long long *S, *T; };
-struct AheadRaw { uint4 v[4]; unsigned a0, a1; unsigned long long s, t; unsigned flags; };  // flags: 1 = tile to count, 2 = extent wanted
+#ifndef DCTZ_COUNT_LEAD
+#define DCTZ_COUNT_LEAD 384u
+#endif
+// units the count ticket may run ahead of the decode ticket: 384 units of 4 tiles = 3 MB of counted bin ids beyond the
+// units the decode warps hold (up to two a warp, 19 MB on a B200); 8 GiB slab on a B200: 1.57-1.58 ms at 192 and 384,
+// 1.58-1.59 at 1024, 1.62 at 2048 units (profiles/README.md)
+constexpr unsigned COUNT_LEAD = DCTZ_COUNT_LEAD;
+struct SplitCfg {
+  static constexpr int DECODE_WARPS = 4, COUNT_WARPS = 4;
+  static constexpr int THREADS = (DECODE_WARPS + COUNT_WARPS) * 32;
+  static constexpr int CTAS_PER_SM = 2;
+  // (DECODE_REGS + COUNT_REGS) * 128 threads * 2 CTAs = 65536 = the register file; the launch gives every thread 128
+  static constexpr unsigned DECODE_REGS = 216, COUNT_REGS = 40;
+};
+static_assert((SplitCfg::DECODE_REGS + SplitCfg::COUNT_REGS) * 128 * SplitCfg::CTAS_PER_SM == 65536, "the register split must fill the register file");
+template <unsigned N> __device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" ::"n"(N)); }
+template <unsigned N> __device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" ::"n"(N)); }
+#ifdef DCTZ_WAIT_STATS
+// diagnostic build (-DDCTZ_WAIT_STATS): [0] decode-warp re-reads of counts not yet published, [1] count-warp looks at a
+// closed lead window, [2] units counted; printed by dctz_gpu_destroy
+__device__ unsigned long long g_wait_stats[3];
+#endif
+
+struct AheadBufs { unsigned *counts, *agg; unsigned long long *S, *T; };
 __device__ __forceinline__ unsigned ld_volatile(const unsigned *p) {
   unsigned v;
   asm volatile("ld.volatile.global.u32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
@@ -1726,110 +1760,114 @@ __device__ __forceinline__ unsigned long long warp_sum_u64(unsigned long long v)
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);
   return v;
 }
-struct AheadExtents {
-  typedef AheadRaw Raw;
-#ifndef DCTZ_AHEAD_DIST
-#define DCTZ_AHEAD_DIST 10
+constexpr unsigned long long AHEAD_LOW48 = 0xFFFFFFFFFFFFull;
+
+// The count warpgroup's loop (one warp).  Returns when the count ticket has passed the last unit.
+__device__ __forceinline__ void count_units(const uint8_t *__restrict__ bins, unsigned long long nblk_full, unsigned ntiles, unsigned batch,
+                                            unsigned nunits, AheadBufs b, unsigned *count_ticket, const unsigned *decode_ticket, int lane) {
+  const unsigned long long pol = policy_evict_last();
+  unsigned lead_end = 0;  // units below it may be counted: decode tickets taken (as last read) + COUNT_LEAD
+#ifdef DCTZ_WAIT_STATS
+  unsigned long long n_wait = 0, n_units = 0;
 #endif
-  static constexpr unsigned AHEAD = DCTZ_AHEAD_DIST;  // tiles between the count cursor and the extent cursor (>= batch + 3)
-  static constexpr unsigned long long LOW48 = 0xFFFFFFFFFFFFull;
+  for (;;) {
+    unsigned u = 0;
+    if (lane == 0) u = ticket_next(count_ticket);
+    u = __shfl_sync(0xFFFFFFFFu, u, 0);
+    if (u >= nunits) break;
+    while (u >= lead_end) {
+      lead_end = ld_volatile(decode_ticket) + COUNT_LEAD;
+      if (u < lead_end) break;
+#ifdef DCTZ_WAIT_STATS
+      n_wait++;
+#endif
+      // the decoders take ~90 units per microsecond on a B200; sleep about as long as the window needs to open, so
+      // that a thousand waiting warps do not hammer the decode ticket's line
+      const unsigned short_by = u + 1u - lead_end;
+      __nanosleep(short_by < 256u ? 64u + 16u * short_by : 4096u);
+    }
+    const unsigned t0 = u * batch, t1 = (t0 + batch < ntiles) ? t0 + batch : ntiles;
+    unsigned sum = 0;
+    for (unsigned t = t0; t < t1; t++) {
+      const unsigned long long first = (unsigned long long)t * WTILE;
+      const unsigned rows = (nblk_full - first < (unsigned long long)WTILE) ? (unsigned)(nblk_full - first) : (unsigned)WTILE;
+      const uint4 *p = reinterpret_cast<const uint4 *>(bins + first * BLK);
+      uint4 v[4];
+#pragma unroll
+      for (int i = 0; i < 4; i++) {
+        const unsigned chunk = i * 32 + lane;  // 16-byte chunk of the tile; 4 chunks per block
+        v[i] = (chunk < rows * 4u) ? ldg_hint(p + chunk, pol) : make_uint4(0u, 0u, 0u, 0u);  // (zero words hold no marker)
+      }
+      unsigned cnt = 0;
+#pragma unroll
+      for (int i = 0; i < 4; i++) {
+        const unsigned x0 = (lane & 3) ? v[i].x : (v[i].x & 0xFFFFFF00u);  // byte 0 of a block is the DC marker (chunk & 3 == lane & 3)
+        cnt += __popc(ff_flags(x0)) + __popc(ff_flags(v[i].y)) + __popc(ff_flags(v[i].z)) + __popc(ff_flags(v[i].w));
+      }
+      cnt = __reduce_add_sync(0xFFFFFFFFu, cnt);
+      if (lane == 0) asm volatile("st.volatile.global.u32 [%0], %1;\n" ::"l"(b.counts + t), "r"(0x80000000u | cnt) : "memory");
+      sum += cnt;
+    }
+    if (lane == 0) {
+      asm volatile("st.volatile.global.u32 [%0], %1;\n" ::"l"(b.agg + u), "r"(0x80000000u | sum) : "memory");
+      const unsigned long long contrib = (1ull << 48) | (unsigned long long)sum;
+      atomicAdd(b.S + (u >> 6), contrib);
+      atomicAdd(b.T + (u >> 11), contrib);
+    }
+#ifdef DCTZ_WAIT_STATS
+    n_units++;
+#endif
+  }
+#ifdef DCTZ_WAIT_STATS
+  if (lane == 0) { atomicAdd(&g_wait_stats[1], n_wait); atomicAdd(&g_wait_stats[2], n_units); }
+#endif
+}
+
+// The decode warpgroup's tile sequence (advance) and extent source (load / finish) for decompress_tiles.  Units come from
+// the decode ticket, the first one too (a statically assigned first unit could belong to a CTA that is not resident yet).
+// Unit u is tiles [u * batch, (u + 1) * batch); a warp takes its units whole and in increasing order, so the extent of a
+// unit's first tile is finished before those of its other tiles, and the super-group sums it has added up stay valid.
+struct CountedExtents {
+  struct Raw { unsigned c, k, u, a0, a1; unsigned long long s, t; };  // loaded values, untouched until finish()
   static __device__ __forceinline__ Raw none() {
     Raw r;
-#pragma unroll
-    for (int i = 0; i < 4; i++) r.v[i] = make_uint4(0u, 0u, 0u, 0u);
-    r.a0 = r.a1 = 0x80000000u; r.s = r.t = 0ull; r.flags = 0u;
+    r.c = 0x80000000u; r.k = 0; r.u = 0; r.a0 = r.a1 = 0x80000000u; r.s = r.t = 0ull;
     return r;
   }
-  const uint8_t *bins;
-  unsigned long long nblk_full, n_limit, pol;
-  unsigned ntiles, batch, nunits, base;
   AheadBufs b;
+  unsigned long long n_limit;
   unsigned *corrupt_flag, *counter;
-  unsigned pend;                                       // lane 0: the ticket requested for the unit after the one being counted
-  unsigned c_start, c_off, c_sum, c_pos, c_units;      // count cursor: unit start, tile in unit, outliers so far, tiles / units so far
-  bool c_done;
-  unsigned ring_cnt, ring_start;                       // lane p & 31: outliers of the warp's p-th tile; lane k & 31: first tile of its k-th unit
-  unsigned p_unit, p_off;                              // process cursor (advance)
-  unsigned e_unit, e_off, e_pos, e_within;             // extent cursor (finish)
-  unsigned long long e_base;
-  unsigned t_upto;                                     // super-groups [0, t_upto) are complete and summed in t_sum
+  unsigned ntiles, batch, nunits;
+  unsigned pend, next, end;          // sequence: lane 0 holds the ticket requested for the unit after [next, end)
+  unsigned long long u_base;         // first outlier of the unit whose extents are being finished
+  unsigned t_upto;                   // super-groups [0, t_upto) are complete and summed in t_sum
   unsigned long long t_sum;
+#ifdef DCTZ_WAIT_STATS
+  unsigned long long n_spin;
+#endif
 
-  __device__ __forceinline__ void open_unit(unsigned start, int lane) {
-    c_start = start; c_off = 0; c_sum = 0;
-    if ((unsigned)lane == (c_units & 31u)) ring_start = start;
-    c_units++;
-    c_done = start >= ntiles;
-  }
-  __device__ __forceinline__ void load_count(Raw &r, int lane) const {
-    const unsigned t = c_start + c_off;
-    if (c_done || t >= ntiles) return;
-    r.flags |= 1u;
-    const unsigned long long first = (unsigned long long)t * WTILE;
-    const unsigned rows = (nblk_full - first < (unsigned long long)WTILE) ? (unsigned)(nblk_full - first) : (unsigned)WTILE;
-    const uint4 *p = reinterpret_cast<const uint4 *>(bins + first * BLK);
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      const unsigned chunk = i * 32 + lane;  // 16-byte chunk of the tile; 4 chunks per block
-      r.v[i] = (chunk < rows * 4u) ? ldg_hint(p + chunk, pol) : make_uint4(0u, 0u, 0u, 0u);  // (zero words hold no marker)
-    }
-  }
-  __device__ __forceinline__ void finish_count(const Raw &r, int lane) {
-    if (!(r.flags & 1u)) return;
-    unsigned cnt = 0;
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      const unsigned chunk = i * 32 + lane;
-      const unsigned x0 = (chunk & 3u) ? r.v[i].x : (r.v[i].x & 0xFFFFFF00u);  // byte 0 of a block is the DC marker
-      cnt += __popc(ff_flags(x0)) + __popc(ff_flags(r.v[i].y)) + __popc(ff_flags(r.v[i].z)) + __popc(ff_flags(r.v[i].w));
-    }
-    cnt = __reduce_add_sync(0xFFFFFFFFu, cnt);
-    if ((unsigned)lane == (c_pos & 31u)) ring_cnt = cnt;
-    c_sum += cnt; c_pos++; c_off++;
-    if (c_off == batch || c_start + c_off >= ntiles) {  // the unit is counted: publish it, open the next one
-      const unsigned u = c_start / batch;
-      if (lane == 0) {
-        asm volatile("st.volatile.global.u32 [%0], %1;\n" ::"l"(b.agg + u), "r"(0x80000000u | c_sum) : "memory");
-        const unsigned long long contrib = (1ull << 48) | (unsigned long long)c_sum;
-        atomicAdd(b.S + (u >> 6), contrib);
-        atomicAdd(b.T + (u >> 11), contrib);
-      }
-      const unsigned start = (base + __shfl_sync(0xFFFFFFFFu, pin_here(pend), 0)) * batch;
-      if (lane == 0) pend = ticket_next(counter);
-      open_unit(start, lane);
-    }
-  }
-  __device__ __forceinline__ void init(const uint8_t *bins_, unsigned long long nblk_full_, unsigned ntiles_, unsigned batch_, AheadBufs bufs,
-                                       unsigned long long n_limit_, unsigned *corrupt_flag_, unsigned *ticket_counter, unsigned warp_global,
-                                       unsigned nwarps_grid, int lane) {
-    bins = bins_; nblk_full = nblk_full_; ntiles = ntiles_; batch = batch_; nunits = (ntiles_ + batch_ - 1) / batch_; b = bufs;
-    n_limit = n_limit_; corrupt_flag = corrupt_flag_; counter = ticket_counter; base = 0u;
-    (void)warp_global; (void)nwarps_grid;
-    pol = policy_evict_last();
-    pend = 0; c_pos = 0; c_units = 0; ring_cnt = 0; ring_start = 0xFFFFFFFFu;
-    p_unit = 0; p_off = 0; e_unit = 0; e_off = 0; e_pos = 0; e_within = 0; e_base = 0ull; t_upto = 0; t_sum = 0ull;
-    // EVERY unit comes from the ticket counter, the first one too: a unit below a ticketed one then belongs to a warp that
-    // is running (a statically assigned first unit could belong to a CTA that is not resident yet -- two such kernels of two
-    // contexts sharing the device would wait for each other's missing CTAs for ever)
+  __device__ __forceinline__ void init(unsigned ntiles_, unsigned batch_, AheadBufs bufs, unsigned long long n_limit_, unsigned *corrupt_flag_,
+                                       unsigned *ticket_counter, int lane) {
+    b = bufs; ntiles = ntiles_; batch = batch_; nunits = (ntiles_ + batch_ - 1) / batch_;
+    n_limit = n_limit_; corrupt_flag = corrupt_flag_; counter = ticket_counter;
+    u_base = 0ull; t_upto = 0; t_sum = 0ull;
+#ifdef DCTZ_WAIT_STATS
+    n_spin = 0;
+#endif
+    pend = 0;
     if (lane == 0) pend = ticket_next(counter);
-    {
-      const unsigned start = __shfl_sync(0xFFFFFFFFu, pin_here(pend), 0) * batch;
-      if (lane == 0) pend = ticket_next(counter);
-      open_unit(start, lane);
-    }
-    for (unsigned i = 0; i < AHEAD; i++) {  // (latency exposed AHEAD times, once per warp and launch)
-      Raw r = none();
-      load_count(r, lane);
-      finish_count(r, lane);
-    }
+    next = end = 0;
   }
-  __device__ __forceinline__ unsigned advance(int) {  // warp-uniform: the next tile to process
-    const unsigned st = __shfl_sync(0xFFFFFFFFu, ring_start, (int)(p_unit & 31u));
-    if (st >= ntiles) return 0xFFFFFFFFu;
-    const unsigned t = st + p_off;
-    if (t >= ntiles) return 0xFFFFFFFFu;
-    if (++p_off == batch) { p_off = 0; p_unit++; }
-    return t;
+  __device__ __forceinline__ unsigned advance(int lane) {  // warp-uniform: the next tile to process
+    if (next >= end) {
+      const unsigned start = __shfl_sync(0xFFFFFFFFu, pin_here(pend), 0) * batch;
+      if (start >= ntiles) { next = end = ntiles; return 0xFFFFFFFFu; }  // (no further ticket)
+      if (lane == 0) pend = ticket_next(counter);
+      next = start;
+      end = start + batch;
+    }
+    if (next >= ntiles) return 0xFFFFFFFFu;
+    return next++;
   }
   // what unit u's offset needs: lanes hold the units of its group below it, the groups of its super-group below its
   // group, and a window of the not yet summed super-groups below its super-group
@@ -1849,42 +1887,43 @@ struct AheadExtents {
     if (wi < h) { const unsigned want = nunits - (wi << 11) < 2048u ? nunits - (wi << 11) : 2048u; ok = ok && (unsigned)(r.t >> 48) == want; }
     return __all_sync(0xFFFFFFFFu, ok);
   }
-  __device__ __forceinline__ Raw load(unsigned /*nn: the tile whose extent the matching finish() returns*/, int lane) const {
+  __device__ __forceinline__ void load_counts(Raw &r, int lane) const {  // lanes < k: earlier tiles of the unit; lane k: the tile
+    r.c = ((unsigned)lane <= r.k) ? ld_volatile(b.counts + r.u * batch + (unsigned)lane) : 0x80000000u;
+  }
+  __device__ __forceinline__ Raw load(unsigned t, int lane) const {
     Raw r = none();
-    r.flags = 2u;
-    load_count(r, lane);
-    if (e_off == 0) {  // its extent starts a unit: the unit's offset is looked up
-      const unsigned u = __shfl_sync(0xFFFFFFFFu, ring_start, (int)(e_unit & 31u)) / batch;
-      load_lookback(r, u, t_upto, lane);
-    }
+    r.u = t / batch;
+    r.k = t - r.u * batch;
+    load_counts(r, lane);
+    if (r.k == 0) load_lookback(r, r.u, t_upto, lane);  // the tile starts a unit: the unit's offset is looked up
     return r;
   }
   __device__ __forceinline__ Extent finish(Raw &r, int lane) {
-    finish_count(r, lane);
-    Extent e;
-    e.base = 0; e.total = 0; e.bad = false;
-    if (!(r.flags & 2u)) return e;
-    if (e_off == 0) {
-      const unsigned u = __shfl_sync(0xFFFFFFFFu, ring_start, (int)(e_unit & 31u)) / batch;
-      const unsigned h = u >> 11;
-      for (;;) {  // (complete at the first look unless a warp has fallen AHEAD tiles behind the others)
+    r.c = pin_here(r.c);  // first use of the loaded values: here, at the end of the iteration
+    if (r.k == 0) {
+      const unsigned u = r.u, h = u >> 11;
+      r.a0 = pin_here(r.a0);
+      for (;;) {  // (complete at the first look unless the counters have fallen behind)
         while (!lookback_complete(r, u, t_upto, lane)) load_lookback(r, u, t_upto, lane);
         if (t_upto + 32u >= h) break;
-        t_sum += warp_sum_u64(r.t & LOW48);  // more than 32 new super-groups (a very large slab's first look): next window
+        t_sum += warp_sum_u64(r.t & AHEAD_LOW48);  // more than 32 new super-groups (a very large slab's first look): next window
         t_upto += 32u;
         load_lookback(r, u, t_upto, lane);
       }
-      t_sum += warp_sum_u64(r.t & LOW48);
+      t_sum += warp_sum_u64(r.t & AHEAD_LOW48);
       t_upto = h;
       const unsigned within = __reduce_add_sync(0xFFFFFFFFu, (r.a0 & 0x7FFFFFFFu) + (r.a1 & 0x7FFFFFFFu));
-      e_base = t_sum + warp_sum_u64(r.s & LOW48) + within;
-      e_within = 0;
+      u_base = t_sum + warp_sum_u64(r.s & AHEAD_LOW48) + within;
     }
-    e.total = __shfl_sync(0xFFFFFFFFu, ring_cnt, (int)(e_pos & 31u));
-    e.base = e_base + e_within;
-    e_within += e.total;
-    e_pos++;
-    if (++e_off == batch) { e_off = 0; e_unit++; }
+    while (!__all_sync(0xFFFFFFFFu, r.c >> 31)) {  // a count not yet published
+#ifdef DCTZ_WAIT_STATS
+      n_spin++;
+#endif
+      load_counts(r, lane);
+    }
+    Extent e;
+    e.total = __shfl_sync(0xFFFFFFFFu, r.c, (int)r.k) & 0x7FFFFFFFu;
+    e.base = u_base + __reduce_add_sync(0xFFFFFFFFu, ((unsigned)lane < r.k) ? (r.c & 0x7FFFFFFFu) : 0u);
     e.bad = e.base + e.total > n_limit;
     if (e.bad) { e.total = 0u; *corrupt_flag = 1u; }
     return e;
@@ -2158,24 +2197,27 @@ __device__ __forceinline__ void decompress_tiles(const uint8_t *__restrict__ bin
   }
 }
 
-// AHEAD = false: extents from the pre-pass (k_count_bins + k_scan_groups).  AHEAD = true: no pre-pass, the warps count
-// ahead and look the offsets up (AheadExtents); `counts` / `group_prefix` / `chunk_prefix` then carry AheadBufs' agg / S / T
+// AHEAD = false: extents from the pre-pass (k_count_bins + k_scan_groups), `counts` are its per-tile counts.  AHEAD = true: no
+// pre-pass, a count warpgroup publishes the counts while the decode warpgroup runs the tile loop (count_units /
+// CountedExtents); `counts`, `unit_counts`, `group_prefix` and `chunk_prefix` then carry AheadBufs' counts / agg / S / T
 // (zeroed by the host before the launch) and the last CTA writes the number of outliers the full blocks hold to
 // `n_outliers_total` (the tail block's offset).
 template <typename T, bool QT, bool AHEAD>
-__global__ void __launch_bounds__(DecompressCfg<T, QT>::THREADS, DecompressCfg<T, QT>::CTAS_PER_SM)
+__global__ void __launch_bounds__(AHEAD ? SplitCfg::THREADS : DecompressCfg<T, QT>::THREADS, AHEAD ? SplitCfg::CTAS_PER_SM : DecompressCfg<T, QT>::CTAS_PER_SM)
 k_decompress(const uint8_t *__restrict__ bins, const float *__restrict__ dc_in, const float *__restrict__ ac_in,
              const T *__restrict__ qtable, unsigned long long nblk_full, T bin_width, T sf, QtConsts<T> qk,
-             const __grid_constant__ CUtensorMap tmap_out, unsigned *counts,
+             const __grid_constant__ CUtensorMap tmap_out, unsigned *counts, unsigned *unit_counts,
              unsigned long long *group_prefix, unsigned long long *chunk_prefix,
              unsigned long long *n_outliers_total, unsigned long long n_limit, TileControl *ctl,
              unsigned *corrupt_flag, int dc_aligned16, unsigned batch, int l2_hints) {
   typedef DecompressCfg<T, QT> Cfg;
+  constexpr int THREADS = AHEAD ? SplitCfg::THREADS : Cfg::THREADS;
   extern __shared__ unsigned char smem_raw[];
   __shared__ __align__(8) unsigned long long s_mbar[Cfg::WARPS];
   __shared__ T s_qt[QT ? BLK : 1];
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const bool decoder = warp < Cfg::WARPS;  // AHEAD: warps Cfg::WARPS.. are the count warpgroup
   unsigned char *smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   __shared__ __align__(16) T center[256];  // static: its address is an immediate of the lookups
   unsigned char *wsm = smem + warp * Cfg::WARP_BYTES;
@@ -2185,35 +2227,44 @@ k_decompress(const uint8_t *__restrict__ bins, const float *__restrict__ dc_in, 
   // floats are put in the upper half of the stage and expanded in place from the bottom.  Tiles with more than
   // FAST_MAX outliers (double) and QT tiles (whose outliers are rescaled with a per-position table entry,
   // dctz-decomp-lib.c:404-409) take the per-lane conversion path.
-  const unsigned mb = smem_u32(&s_mbar[warp]);
+  const unsigned mb = smem_u32(&s_mbar[decoder ? warp : 0]);
 
   // bin centres: gen_bins / gen_bins_f (binning.c:19-22, 39-42): centre = (int multiple) * bin_width.  The de-scale
   // (x * sf, dctz-decomp-lib.c:494-511) is folded into the coefficients -- the inverse transform is linear, the
   // result moves by ~1 ulp -- so the table holds centre * sf.
-  for (int i = threadIdx.x; i < 256; i += Cfg::THREADS) center[i] = center_coefficient<T>((unsigned)i, bin_width, sf);
+  for (int i = threadIdx.x; i < 256; i += THREADS) center[i] = center_coefficient<T>((unsigned)i, bin_width, sf);
   if (QT && threadIdx.x < BLK) s_qt[threadIdx.x] = qtable[threadIdx.x];
-  if (lane == 0) { mbar_init(mb, 1); fence_mbar_init(); }
+  if (decoder && lane == 0) { mbar_init(mb, 1); fence_mbar_init(); }
   __syncthreads();  // the only CTA-wide barrier before the epilogue
 
   unsigned phase = 0;
+  const unsigned ntiles = (unsigned)((nblk_full + WTILE - 1) / WTILE);
   if constexpr (AHEAD) {
-    AheadExtents ah;
     AheadBufs ab;
-    ab.agg = counts; ab.S = group_prefix; ab.T = chunk_prefix;
-    const unsigned ntiles = (unsigned)((nblk_full + WTILE - 1) / WTILE);
-    ah.init(bins, nblk_full, ntiles, batch, ab, n_limit, corrupt_flag, &ctl->ticket, blockIdx.x * Cfg::WARPS + warp, gridDim.x * Cfg::WARPS, lane);
-    decompress_tiles<T, QT>(bins, dc_in, ac_in, nblk_full, sf, qk, &tmap_out, n_limit, dc_aligned16, wsm, mb, center, s_qt, ah, ah, lane, phase,
-                            l2_hints);
-    bulk_wait_all();
-    if (lane == 0) (void)pin_here(ah.pend);  // (as below)
+    ab.counts = counts; ab.agg = unit_counts; ab.S = group_prefix; ab.T = chunk_prefix;
+    const unsigned nunits = (ntiles + batch - 1) / batch;
+    if (!decoder) {
+      setmaxnreg_dec<SplitCfg::COUNT_REGS>();
+      count_units(bins, nblk_full, ntiles, batch, nunits, ab, &ctl->count_ticket, &ctl->ticket, lane);
+    } else {
+      setmaxnreg_inc<SplitCfg::DECODE_REGS>();
+      CountedExtents ce;
+      ce.init(ntiles, batch, ab, n_limit, corrupt_flag, &ctl->ticket, lane);
+      decompress_tiles<T, QT>(bins, dc_in, ac_in, nblk_full, sf, qk, &tmap_out, n_limit, dc_aligned16, wsm, mb, center, s_qt, ce, ce, lane, phase,
+                              l2_hints);
+      bulk_wait_all();
+      if (lane == 0) (void)pin_here(ce.pend);  // (as below)
+#ifdef DCTZ_WAIT_STATS
+      if (lane == 0) atomicAdd(&g_wait_stats[0], ce.n_spin);
+#endif
+    }
   } else {
     const unsigned long long n_scan = __ldg(n_outliers_total);
     ScannedExtents ext;
     ext.counts = counts; ext.group_prefix = group_prefix; ext.chunk_prefix = chunk_prefix; ext.n_limit = n_limit; ext.corrupt_flag = corrupt_flag;
     TileSeq seq;
     // l2_hints bit 2: from the last tile down -- what the pre-pass read last (with evict_last) is what L2 still holds
-    const unsigned ntiles_ = (unsigned)((nblk_full + WTILE - 1) / WTILE);
-    seq.init(&ctl->ticket, blockIdx.x * Cfg::WARPS + warp, gridDim.x * Cfg::WARPS, batch, lane, (l2_hints & 4) ? ntiles_ - 1u : 0u);
+    seq.init(&ctl->ticket, blockIdx.x * Cfg::WARPS + warp, gridDim.x * Cfg::WARPS, batch, lane, (l2_hints & 4) ? ntiles - 1u : 0u);
     decompress_tiles<T, QT>(bins, dc_in, ac_in, nblk_full, sf, qk, &tmap_out, n_scan < n_limit ? n_scan : n_limit, dc_aligned16, wsm, mb, center,
                             s_qt, seq, ext, lane, phase, l2_hints);
     bulk_wait_all();
@@ -2227,16 +2278,15 @@ k_decompress(const uint8_t *__restrict__ bins, const float *__restrict__ dc_in, 
   if (threadIdx.x == 0) {
     const unsigned prev = atomicAdd(&ctl->done, 1u);
     s_last = (prev == gridDim.x - 1);
-    if (s_last) { ctl->ticket = 0u; ctl->done = 0u; }
+    if (s_last) { ctl->ticket = 0u; ctl->count_ticket = 0u; ctl->done = 0u; }
   }
   if constexpr (AHEAD) {
     __syncthreads();
     if (s_last && warp == 0) {  // every unit has been published: the full blocks' outliers = the sum over the super-groups
       __threadfence();
-      const unsigned ntiles = (unsigned)((nblk_full + WTILE - 1) / WTILE);
       const unsigned nunits = (ntiles + batch - 1) / batch, nsuper = (nunits + 2047u) >> 11;
       unsigned long long tot = 0ull;
-      for (unsigned w = lane; w < nsuper; w += 32) tot += ld_volatile(chunk_prefix + w) & AheadExtents::LOW48;
+      for (unsigned w = lane; w < nsuper; w += 32) tot += ld_volatile(chunk_prefix + w) & AHEAD_LOW48;
       tot = warp_sum_u64(tot);
       if (lane == 0) *n_outliers_total = tot;
     }
